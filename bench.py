@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (N>1: launched by torch.distributed.run)
   python bench.py --impl reference --gpus N --steps K --warmup W
+  python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   (+ DIR/<name>.npy: results of the last timed step)
 
 A "step" is one pass of the hot path over the synthetic batch: K1 ragged spline resample of every
 history -> (N>1: one NCCL all-gather of the resampled rows) -> K2 all-pairs GEMM-form filter (tcgen05
@@ -224,6 +225,36 @@ def edge_checksums(a, b, d, n):
     return {"edges": int(len(a)), "sum_keys_mod_2_64": ck, "xor_distance_bits": cd}
 
 
+DUMP_EDGES = 3 << 19   # 1.5 Mi edges x 4 arrays x 8 bytes = 48 MiB
+DUMP_ROWS = 4096
+
+
+class DeviceRows:
+    """A [n, k] float64 matrix in device memory owned by the library, visible to torch without a copy."""
+
+    def __init__(self, ptr, n, k):
+        self.__cuda_array_interface__ = {"shape": (n, k), "typestr": "<f8", "data": (ptr, False), "strides": None,
+                                         "version": 3}
+
+
+def dump_outputs(out_dir, a, b, d, rows):
+    """--dump-outputs: the edge list (a, b, d) and the resampled rows (a [n, K] float64 CUDA tensor) as float64 .npy
+    files in out_dir. Longer lists and larger matrices are represented by fixed samples (seed 0) whose positions are
+    stored beside them, so that two builds given the same arguments can be compared file for file. At most 58 MiB
+    (K = 300)."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    m, n = len(a), rows.shape[0]
+    rng = np.random.default_rng(0)
+    pos = np.sort(rng.choice(m, DUMP_EDGES, replace=False)) if m > DUMP_EDGES else np.arange(m)
+    ridx = np.sort(rng.choice(n, DUMP_ROWS, replace=False)) if n > DUMP_ROWS else np.arange(n)
+    sample = rows[torch.from_numpy(ridx).to(rows.device)].cpu().numpy()
+    out = {"edge_count": np.array([m]), "edge_sample_position": pos, "edge_a": a[pos], "edge_b": b[pos],
+           "edge_distance": d[pos], "spline_row_index": ridx, "spline_rows": sample}
+    for name, arr in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(arr, dtype=np.float64))
+
+
 def verify_run(args, hc, sc, world, rank, dev, n, P, variant, stream_mode, level, gloo=None):
     """One more, untimed, pass of exactly the path that was timed (same context, same variant, same sharding), then:
       (i)   every rank's list sorted and unique; the union of the ranks' lists unique;
@@ -419,17 +450,25 @@ def run_ours(args, wl, wl_name):
            "edges": 0, "survivors": 0}
 
     streamed = {"edges": 0, "chunks": 0}
+    # what the latest resident step handed its caller (--dump-outputs): the shard counts and full rows (N > 1) and,
+    # streamed, the edge chunks (collected only while "chunks" is present)
+    last = {}
 
     def sink(a, b, d):
         streamed["edges"] += len(a)
         streamed["chunks"] += 1
+        if "chunks" in last:
+            last["chunks"].append((a, b, d))
 
     def step_resident(record):
+        if args.dump_outputs and args.stream:
+            last["chunks"] = []
         if world > 1:
             if overlapped:
-                ne, counts, offs, _ = sc.run_overlapped(n, P, THR)
+                ne, counts, offs, full = sc.run_overlapped(n, P, THR)
             else:
-                ne, counts, offs, _ = sc.run(n, P, THR, variant, sink=sink if args.stream else None)
+                ne, counts, offs, full = sc.run(n, P, THR, variant, sink=sink if args.stream else None)
+            last["counts"], last["full"] = counts, full
             tot = sum(counts)
         else:
             hc.resample(P)
@@ -511,8 +550,29 @@ def run_ours(args, wl, wl_name):
         ms = float(t.item())
     value = total_pairs * args.steps / (ms * 1e-3)
 
+    if args.dump_outputs:
+        # what the last timed step computed, read back after the timed region
+        if args.stream:
+            ch = last.pop("chunks")
+            a, b, d = (np.concatenate([c[k] for c in ch]) if ch else np.zeros(0, dtype=(np.uint32, np.uint32, np.float64)[k])
+                       for k in range(3))
+        else:
+            a, b, d = hc.get_edges()
+        if world > 1:
+            from scema_b200.distributed import gather_edges
+            a, b, d = gather_edges(a, b, d, n, last["counts"], dev)
+        if rank == 0:
+            if world > 1:
+                rows = last["full"]
+            else:
+                n_rows, K_rows, ptr = hc.spline_info()
+                rows = torch.as_tensor(DeviceRows(ptr, n_rows, K_rows), device=dev)
+            dump_outputs(args.dump_outputs, a, b, d, rows)
+        if world > 1:
+            dist.barrier()
+
     # ---- end-to-end timing (host buffers)
-    e2e_steps = max(1, min(args.steps, 3))
+    e2e_steps = args.steps
     step_e2e()
     barrier()
     ev0.record(stream)
@@ -770,7 +830,12 @@ def main():
                          "(full: 1000 rows and 64 tiles of 1024 x 1024, the config-5 checks of SURVEY 8d)")
     ap.add_argument("--stream", type=int, default=-1,
                     help="1: edges leave the device chunk by chunk through scema_compare_stream (default for c5), 0: one-shot compare")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the edge list and resampled rows of the last timed step to DIR/<name>.npy (float64, "
+                         "fixed seeded samples when larger than ~50 MB) so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     wl = dict(WORKLOADS[args.workload])
     if args.stream < 0:
