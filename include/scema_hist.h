@@ -267,7 +267,9 @@ int scema_last_audit(scema_ctx *ctx, uint64_t out[2]);
  * sliced products, slices = 1: a_hi.b_hi only, with the wider guard band folded in), operand_a_host /
  * operand_b_host (n_pad * 256 bytes each, may be NULL) the fp16 operand copies as they sit in memory:
  * blocks of 128 rows, each [hi slice | lo slice] of 128 rows x 128 bytes, 16-byte chunk c of row r
- * stored at chunk c ^ (r & 7). */
+ * stored at chunk c ^ (r & 7). slices = 3: the projected filter (16 <= k <= 60); the operand copies are then
+ * n_pad * 32 bytes each: blocks of 128 rows x 32 bytes, 16 fp16 per row (11 basis coordinates, the residual norm,
+ * 4 fold columns), 16-byte chunk c of row r stored at chunk c ^ ((r >> 2) & 1). */
 int scema_tc_debug(scema_ctx *ctx, double threshold, uint32_t slices, float *acc_host, uint64_t ld,
                    void *operand_a_host, void *operand_b_host);
 /* The column means the tcgen05 filter subtracted from its operand copies (centre_host[k], k = columns of the rows;
@@ -282,6 +284,17 @@ int scema_tc_last_plan(scema_ctx *ctx, uint64_t plan[6]);
  * or -1 (SCEMA_PAIRS_EXACT), *centred = whether the tcgen05 copies are centred, *est_survivors = queue entries expected. */
 int scema_tc_choose(uint64_t pairs, uint32_t k, const uint64_t counts[5], uint64_t sample, uint64_t mem_budget, int *choice,
                     int *centred, uint64_t *est_survivors);
+/* The same with a sixth count, the pairs of the sample that would survive the projected filter (16-column copies:
+ * coordinates in a basis of the sample's leading principal directions plus the residual norm); *choice = 3 selects it. */
+int scema_tc_choose_projected(uint64_t pairs, uint32_t k, const uint64_t counts[6], uint64_t sample, uint64_t mem_budget,
+                              int *choice, int *centred, uint64_t *est_survivors);
+/* The projected filter's basis as host logic: from the second moments moments[k * k] of the centred sample, 11 orthonormal
+ * rows basis[11 * 60] (row-major, zero beyond k) and *delta = |B B^T - I|_F. SCEMA_ERR_INVALID when k is outside
+ * [16, 60], the moments are not finite or delta exceeds 2^-32 (the filter then keeps its 64-column copies). */
+int scema_tc_basis(const double *moments, uint32_t k, double *basis, double *delta);
+/* The projected filter in the last automatic choice: out = {pairs of the survivor-density sample that would survive it,
+ * 1 if the operand copies are the projected ones}. */
+int scema_tc_last_projection(scema_ctx *ctx, uint64_t out[2]);
 /* Ranges of histories the host-buffer pipeline of scema_cluster would use for a batch of n (host logic only):
  * bounds[0] = 0 < ... < bounds[*n_ranges] = n, at most 16 ranges, every inner boundary a multiple of 2048. */
 int scema_pipeline_plan(uint64_t n, uint64_t *bounds, uint32_t cap, uint32_t *n_ranges);

@@ -77,6 +77,9 @@ def lib():
         "scema_tc_centre": (i32, [vp, vp]),
         "scema_tc_last_plan": (i32, [vp, vp]),
         "scema_tc_choose": (i32, [u64, u32, vp, u64, u64, P(i32), P(i32), P(u64)]),
+        "scema_tc_choose_projected": (i32, [u64, u32, vp, u64, u64, P(i32), P(i32), P(u64)]),
+        "scema_tc_basis": (i32, [vp, u32, vp, P(dbl)]),
+        "scema_tc_last_projection": (i32, [vp, vp]),
         "scema_pipeline_plan": (i32, [u64, vp, u32, P(u32)]),
         "scema_multi_create": (i32, [P(vp), vp, i32]),
         "scema_multi_destroy": (None, [vp]),
@@ -119,7 +122,7 @@ EXPORTED = (
     "scema_store_reset scema_store_append scema_store_info scema_store_resample scema_select_rows "
     "scema_set_spline scema_get_spline scema_spline_info scema_compare scema_compare_stream scema_get_edges scema_edges_device "
     "scema_get_degrees scema_cluster scema_nearest scema_write_similar_hist scema_reduce_edges scema_reduce_calls scema_reduce_dir "
-    "scema_last_timings scema_last_counters scema_kernel_launches scema_last_audit scema_fp64_peak scema_k1_tune scema_tc_debug scema_tc_plan scema_tc_shard_begin scema_tc_shard_stats scema_tc_shard_finish scema_tc_shard_check scema_tc_shard_commit scema_tc_centre scema_tc_last_plan scema_tc_choose scema_pipeline_plan scema_synth_offsets "
+    "scema_last_timings scema_last_counters scema_kernel_launches scema_last_audit scema_fp64_peak scema_k1_tune scema_tc_debug scema_tc_plan scema_tc_shard_begin scema_tc_shard_stats scema_tc_shard_finish scema_tc_shard_check scema_tc_shard_commit scema_tc_centre scema_tc_last_plan scema_tc_choose scema_tc_choose_projected scema_tc_basis scema_tc_last_projection scema_pipeline_plan scema_synth_offsets "
     "scema_multi_create scema_multi_destroy scema_multi_last_error scema_multi_devices scema_multi_context scema_multi_cluster "
     "scema_multi_compare_rows scema_multi_shard_edges scema_multi_last_ms "
     "scema_synth_histories_device scema_synth_rows_device scema_synth_histories_model_device scema_synth_rows_model_device scema_ingest_last_error scema_batch_read_dir "
@@ -222,13 +225,29 @@ class Batch:
 
 def tc_choose(pairs, k, counts, sample, mem_budget):
     """Host logic of the filter choice (scema_tc_choose); counts = survivors of the sample for (one slice, two slices)
-    centred, (one slice, two slices) raw, DMMA. -> (choice, centred, estimated survivors)."""
-    cnt = (C.c_uint64 * 5)(*[int(x) for x in counts])
+    centred, (one slice, two slices) raw, DMMA and, when a sixth is given, the projected filter (choice 3).
+    -> (choice, centred, estimated survivors)."""
+    cnt = (C.c_uint64 * len(counts))(*[int(x) for x in counts])
+    if len(counts) not in (5, 6):
+        raise ValueError("tc_choose: five or six counts")
+    fn = lib().scema_tc_choose_projected if len(counts) == 6 else lib().scema_tc_choose
     ch, cen, est = C.c_int(0), C.c_int(0), C.c_uint64(0)
-    rc = lib().scema_tc_choose(int(pairs), int(k), cnt, int(sample), int(mem_budget), C.byref(ch), C.byref(cen), C.byref(est))
+    rc = fn(int(pairs), int(k), cnt, int(sample), int(mem_budget), C.byref(ch), C.byref(cen), C.byref(est))
     if rc:
         raise ScemaError(rc, "tc_choose")
     return int(ch.value), int(cen.value), int(est.value)
+
+
+def tc_basis(moments):
+    """Host logic of the projected filter's basis (scema_tc_basis): second moments [k, k] of the centred sample ->
+    (basis [11, k], |B B^T - I|_F), or None when the library would keep the 64-column copies."""
+    m = np.ascontiguousarray(moments, dtype=np.float64)
+    k = m.shape[0]
+    out = np.zeros((11, 60), dtype=np.float64)
+    delta = C.c_double(0.0)
+    if lib().scema_tc_basis(_ptr(m), int(k), _ptr(out), C.byref(delta)):
+        return None
+    return out[:, :k].copy(), float(delta.value)
 
 
 class HistCluster:
@@ -442,12 +461,13 @@ class HistCluster:
         return int(self._L.scema_kernel_launches(self._h))
 
     def tc_debug(self, threshold, n, slices=2):
-        """Accumulators and operand copies of the tcgen05 filter over the whole pair matrix (tests only).
-        Returns (acc [n_pad, n_pad] float32, A operand bytes, B operand bytes)."""
+        """Accumulators and operand copies of the tcgen05 filter over the whole pair matrix (tests only); slices = 3:
+        the projected filter (32-byte operand rows). Returns (acc [n_pad, n_pad] float32, A operand bytes, B operand bytes)."""
         n_pad = (n + 255) // 256 * 256
         acc = np.empty((n_pad, n_pad), dtype=np.float32)
-        ha = np.empty(n_pad * 256, dtype=np.uint8)
-        hb = np.empty(n_pad * 256, dtype=np.uint8)
+        row_bytes = 32 if slices == 3 else 256
+        ha = np.empty(n_pad * row_bytes, dtype=np.uint8)
+        hb = np.empty(n_pad * row_bytes, dtype=np.uint8)
         self._ck(self._L.scema_tc_debug(self._h, float(threshold), int(slices), _ptr(acc), n_pad, _ptr(ha), _ptr(hb)))
         return acc, ha, hb
 
@@ -488,11 +508,14 @@ class HistCluster:
         return out
 
     def tc_last_plan(self):
-        """-> dict: pairs of the last survivor-density sample that would survive 1 slice / 2 slices / DMMA, sample size."""
+        """-> dict: pairs of the last survivor-density sample that would survive 1 slice / 2 slices / DMMA / the projected
+        filter, sample size, and whether the projected filter was taken."""
         p = (C.c_uint64 * 6)()
         self._ck(self._L.scema_tc_last_plan(self._h, p))
+        q = (C.c_uint64 * 2)()
+        self._ck(self._L.scema_tc_last_projection(self._h, q))
         return {"one_slice": int(p[0]), "two_slices": int(p[1]), "one_slice_raw": int(p[2]), "two_slices_raw": int(p[3]),
-                "dmma": int(p[4]), "sample": int(p[5])}
+                "dmma": int(p[4]), "sample": int(p[5]), "projected": int(q[0]), "projected_chosen": bool(q[1])}
 
     def k1_tune(self, kernel=-1, wps_ragged=-1, wps_store=-1, flags=-1):
         """Measurement hook of K1 (process-wide): kernel 1 = two chains per lane / 0 = one, resident warps per SM, memory flags."""

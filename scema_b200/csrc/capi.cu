@@ -55,8 +55,10 @@ void scema_destroy(scema_ctx *c)
     c->d_sort_tmp.release();
     c->d_tc_a.release(); c->d_tc_b.release(); c->d_tc_nrm.release(); c->d_tc_misc.release(); c->d_tc_centre.release();
     c->d_tc_perm.release(); c->d_tc_iota.release(); c->d_tc_snrm.release(); c->d_tc_band.release();
+    c->d_tc_basis.release(); c->d_tc_cov.release();
     if (c->h_counters) cudaFreeHost(c->h_counters);
     if (c->h_plan) cudaFreeHost(c->h_plan);
+    if (c->h_tc_cov) cudaFreeHost(c->h_tc_cov);
     for (int k = 0; k < 2; k++) {
         if (c->h_stage_key[k]) cudaFreeHost(c->h_stage_key[k]);
         if (c->h_stage_val[k]) cudaFreeHost(c->h_stage_val[k]);
@@ -475,7 +477,30 @@ int scema_tc_choose(uint64_t pairs, uint32_t k, const uint64_t counts[5], uint64
                     int *centred, uint64_t *est_survivors)
 {
     if (!counts || !choice || !centred || !est_survivors || sample == 0 || k == 0) return SCEMA_ERR_INVALID;
-    tc_choose(pairs, k, counts, sample, mem_budget, tc_chunks_for(k) <= 10, choice, centred, est_survivors);
+    const uint64_t c6[6] = {counts[0], counts[1], counts[2], counts[3], counts[4], 0};
+    tc_choose(pairs, k, c6, sample, mem_budget, tc_chunks_for(k) <= 10, false, choice, centred, est_survivors);
+    return SCEMA_OK;
+}
+
+int scema_tc_choose_projected(uint64_t pairs, uint32_t k, const uint64_t counts[6], uint64_t sample, uint64_t mem_budget, int *choice,
+                              int *centred, uint64_t *est_survivors)
+{
+    if (!counts || !choice || !centred || !est_survivors || sample == 0 || k == 0) return SCEMA_ERR_INVALID;
+    tc_choose(pairs, k, counts, sample, mem_budget, tc_chunks_for(k) <= 10, true, choice, centred, est_survivors);
+    return SCEMA_OK;
+}
+
+int scema_tc_basis(const double *moments, uint32_t k, double *basis, double *delta)
+{
+    if (!moments || !basis || !delta) return SCEMA_ERR_INVALID;
+    return tc_basis_from_moments(moments, k, basis, delta) ? SCEMA_OK : SCEMA_ERR_INVALID;
+}
+
+int scema_tc_last_projection(scema_ctx *c, uint64_t out[2])
+{
+    if (!c || !out) return SCEMA_ERR_INVALID;
+    out[0] = c->tc_plan_counts[5];
+    out[1] = c->tc_proj ? 1u : 0u;
     return SCEMA_OK;
 }
 

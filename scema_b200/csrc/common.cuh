@@ -18,6 +18,8 @@ constexpr int TILE = 128;         // rows per pair-matrix tile side (K2)
 // decisions: pairs per second of the one-slice / two-slice tcgen05 filter (one chunk of 64 columns), the DMMA filter
 // and the filter-free kernel at K = 60, survivors per second of the exact recompute.
 constexpr double RATE_TC1 = 1.4e13, RATE_TC2 = 4.6e12, RATE_DMMA = 2.9e11, RATE_EXACT = 7.0e10, RATE_QUEUE = 1.0e10;
+// the projected (16-column) tcgen05 filter, pairs per second (config 4: 26.9 ms for 5.0e11 pairs, one B200 at 1000 W)
+constexpr double RATE_TCP = 1.86e13;
 constexpr int PANEL_ROWBLOCKS = 16;  // row blocks per scheduling panel (L2 reuse of the B tiles)
 
 // Growable device buffer.
@@ -114,7 +116,11 @@ struct scema_ctx {
 
     // ---- K2 tensor-core filter (SCEMA_PAIRS_TC): fp16 split operands, A- and B-flavoured
     scema::DevBuf d_tc_a, d_tc_b, d_tc_nrm, d_tc_misc, d_tc_centre;  // centre: [K] column means subtracted in the filter copies only
-    uint64_t tc_plan_counts[5] = {0, 0, 0, 0, 0};  // last survivor-density sample (of tc::PLAN_SAMPLE pairs): one / two slices centred, one / two slices raw, DMMA
+    uint64_t tc_plan_counts[6] = {0, 0, 0, 0, 0, 0};  // last survivor-density sample (of tc::PLAN_SAMPLE pairs): one / two slices centred, one / two slices raw, DMMA, projected
+    scema::DevBuf d_tc_basis, d_tc_cov;  // projected filter: basis rows [11][60] (FP64), sample second moments [K][K]
+    double *h_tc_cov = nullptr;          // pinned copy of the second moments
+    bool tc_proj = false;                // operand copies are the projected 16-column image (k_tc_prep_proj)
+    double tc_basis_h[11 * 60] = {};      // the basis on the host (tc::Basis layout), kernel argument of k_tc_prep_proj
     scema::DevBuf d_tc_perm, d_tc_iota, d_tc_snrm, d_tc_band;  // norm-band mode: permutation, sorted squared norms, band plan
     bool tc_band = false, tc_band_wanted = false, tc_band_allowed = false;
     uint64_t tc_for_version = 0, tc_n = 0;
@@ -220,10 +226,13 @@ bool tc_smem_plan(uint32_t nc, uint32_t slices, uint32_t cg, uint32_t *a_bytes, 
                   uint32_t *stage_bytes, uint32_t *data_bytes);
 uint32_t tc_chunks_for(uint32_t K);
 int tc_prepare(scema_ctx *ctx, double thr, uint32_t slices, bool want_band, uint64_t pairs, int *choice, uint64_t *est_survivors);
-void tc_choose(uint64_t pairs, uint32_t K, const uint64_t counts[5], uint64_t sample, uint64_t mem_budget, bool tc_ok, int *choice,
+void tc_choose(uint64_t pairs, uint32_t K, const uint64_t counts[6], uint64_t sample, uint64_t mem_budget, bool tc_ok, bool proj_ok, int *choice,
                int *centred, uint64_t *est_survivors);
 int tc_centre_rows(scema_ctx *ctx, uint64_t r0, uint64_t r1);
-int tc_plan_rows(scema_ctx *ctx, uint64_t r1, uint64_t counts[5]);
+int tc_plan_rows(scema_ctx *ctx, uint64_t r1, uint64_t counts[6], bool proj);
+bool tc_basis_from_moments(const double *cov, uint32_t K, double *basis, double *delta);
+bool tc_proj_possible(uint32_t K);
+int tc_basis_range(scema_ctx *ctx, uint64_t r0, uint64_t r1, bool *ok);
 uint32_t tc_plan_sample_size();
 int tc_shard_begin(scema_ctx *ctx, double thr, uint64_t r0, uint64_t r1, const double **centre_dev);
 int tc_shard_stats(scema_ctx *ctx, const double *centre_dev, const unsigned long long **packet_dev, uint64_t *packet_words);

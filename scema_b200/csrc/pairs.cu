@@ -1258,13 +1258,15 @@ static int compare_begin(scema_ctx *ctx, double thr, int &variant, uint32_t shar
     const uint64_t queue_floor = std::max<uint64_t>(1ull << 20, 32 * n);  // grows with the batch: a context that started small must not mistake a full queue for a wide guard band
     if (variant != SCEMA_PAIRS_EXACT) t_begin(ctx, SCEMA_T_PREP);
     if (variant == SCEMA_PAIRS_TC) {
-        // How many fp16 slices, or another filter altogether? Pinned by SCEMA_TC_SLICES=1|2, otherwise decided from a
-        // sample of the pairs (tc_prepare / tc_choose; the same rows and threshold keep their earlier decision):
-        // survivors of every option estimated in FP64 BEFORE the first launch, so the common case is one pass.
+        // How many fp16 slices, or another filter altogether? Pinned by SCEMA_TC_SLICES=1|2 (3: the projected 16-column
+        // filter), otherwise decided from a sample of the pairs (tc_prepare / tc_choose; the same rows and threshold keep
+        // their earlier decision): survivors of every option estimated in FP64 BEFORE the first launch, so the common
+        // case is one pass.
         static const char *sl_env = getenv("SCEMA_TC_SLICES");
         const int pin = sl_env ? atoi(sl_env) : 0;
-        uint32_t slices = (pin == 1 || pin == 2) ? (uint32_t)pin : 0u;
+        uint32_t slices = (pin >= 1 && pin <= 3) ? (uint32_t)pin : 0u;
         if (slices == 2 && !tc_two_slices_possible(ctx)) slices = 1;  // K > 60: hi slices only
+        if (slices == 3 && !tc_proj_possible(ctx->K)) slices = 1;
         ctx->tc_mode = slices ? 0u : 1u;                              // 1: automatic (compare_panels may change it on overflow)
         // SCEMA_NORM_BAND=1 (one-shot compares only): rows in norm order, tiles beyond the threshold's reach skipped
         const char *band_env = getenv("SCEMA_NORM_BAND");
@@ -1479,15 +1481,21 @@ static int cluster_pipelined_impl(scema_ctx *ctx, const double *steps_host, uint
         if (!rc) rc = tc_stats_rows(ctx, r0, r1, r == 0);
         if (!rc && r == 0) rc = tc_fix_scale(ctx, 6);
         if (!rc && r == 0) {
-            // is the one-slice filter the right one for this data? (sample of the first range; the host waits for
-            // range 0 here, the later copies keep travelling) If not, the ordinary path decides with all rows in hand.
-            uint64_t counts[5];
-            rc = tc_plan_rows(ctx, r1, counts);
+            // is the one-slice filter (64 columns or projected) the right one for this data? (sample of the first range; the
+            // host waits for range 0 here, the later copies keep travelling) If not, the ordinary path decides with all rows
+            // in hand. The basis, like centre and scale, comes from the first range: later rows outside its span land in
+            // the residual coordinate, which costs survivors, never edges.
+            bool proj_ok = tc_proj_possible(ctx->K);
+            if (proj_ok) rc = tc_basis_range(ctx, r0, r1, &proj_ok);
+            uint64_t counts[6];
+            if (!rc) rc = tc_plan_rows(ctx, r1, counts, proj_ok);
             int choice = 1, centred = 1;
             uint64_t est = 0;
             if (!rc) {
-                tc_choose(n * (n - 1) / 2, ctx->K, counts, tc_plan_sample_size(), (uint64_t)ctx->mem_budget, true, &choice, &centred, &est);
-                if (choice != 1 || !centred || est + est / 4 > ctx->cand_cap) { t_end(ctx, SCEMA_T_FILTER); return SCEMA_OK; }
+                tc_choose(n * (n - 1) / 2, ctx->K, counts, tc_plan_sample_size(), (uint64_t)ctx->mem_budget, true, proj_ok, &choice, &centred,
+                          &est);
+                if (!(choice == 3 || (choice == 1 && centred)) || est + est / 4 > ctx->cand_cap) { t_end(ctx, SCEMA_T_FILTER); return SCEMA_OK; }
+                ctx->tc_proj = choice == 3;
             }
         }
         if (!rc) rc = tc_prep_rows(ctx, r0, r1p);

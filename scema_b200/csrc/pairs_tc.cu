@@ -26,6 +26,8 @@
 #include <cub/device/device_radix_sort.cuh>
 #include <type_traits>
 #include <algorithm>
+#include <cmath>
+#include <vector>
 
 namespace scema {
 namespace tc {
@@ -35,6 +37,11 @@ constexpr uint32_t SLICE_BYTES = ROWS * 128;       // 128 rows x 64 fp16, SW128 
 constexpr uint32_t BLOCK_BYTES = 2 * SLICE_BYTES;  // hi | lo
 constexpr uint32_t COLT = 256;                     // B rows (= pair-matrix columns) per tile
 constexpr uint32_t KMAX = 60;                      // data columns per slice (4 more carry the row terms)
+// Projected (narrow) operands: PROJ_R coordinates of the centred row in an orthonormal basis of the sample's leading
+// principal directions, the norm of the residual, 4 fold columns = 16 fp16 = 32 bytes per row, K-major SWIZZLE_32B
+constexpr uint32_t PROJ_R = 11;
+constexpr uint32_t NROW_BYTES = 32;
+constexpr uint32_t NBLOCK_BYTES = ROWS * NROW_BYTES;  // 4 KB per 128-row block
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
@@ -223,6 +230,13 @@ __device__ __forceinline__ uint64_t make_desc(uint32_t smem_addr)
     const uint32_t hi = (1024u >> 4) | (1u << 14) | (2u << 29);
     return ((uint64_t)hi << 32) | (uint64_t)((smem_addr >> 4) & 0x3FFFu);
 }
+// The same for the narrow operands: rows of 32 bytes (K = 16 fp16, exactly one MMA step), 8-row groups 256 bytes apart,
+// layout type 6 = SWIZZLE_32B (16-byte chunk c of row r stored at chunk c ^ ((r >> 2) & 1)).
+__device__ __forceinline__ uint64_t make_desc32(uint32_t smem_addr)
+{
+    const uint32_t hi = (256u >> 4) | (1u << 14) | (6u << 29);
+    return ((uint64_t)hi << 32) | (uint64_t)((smem_addr >> 4) & 0x3FFFu);
+}
 
 struct Args {
     const unsigned char *HA, *HB;  // [n_pad/128][hi|lo][128 rows][128 bytes, 16-byte chunks XOR-swizzled by row & 7]
@@ -265,7 +279,7 @@ struct Smem {
     static constexpr uint32_t B_SLICE = B_ROWS * 128;             // bytes of one slice of a B stage (one chunk)
     static constexpr uint32_t B_STAGE = 2 * B_SLICE;
     static constexpr uint32_t DATA_MAX = 224 * 1024;              // operand tiles: A buffers, then the B ring
-    static constexpr uint32_t MAXST = 8;
+    static constexpr uint32_t MAXST = 16;
     static constexpr uint32_t n_bars = 3 * MAXST + 6;             // full, pfull, empty | a_empty[2] tfull[2] tempty[2]
     static constexpr uint32_t tail = n_bars * 8 + 16 + 1024;      // barriers, TMEM address, slack to align the base to 1024
 };
@@ -273,7 +287,8 @@ struct Smem {
 // WIDE = false: rows of one chunk (K <= 60) with a compile-time shared-memory plan (A double-buffered at a 32 KB
 // stride, B ring behind it); WIDE = true: several chunks per row, plan from tc_launch.
 // BAND = true: rows are sorted by norm and only the band of tiles the triangle inequality cannot rule out is walked.
-template <int CG, bool DBG, bool WIDE, bool BAND>
+// NARROW = true: projected 16-column operands (k_tc_prep_proj), 4 KB per 128-row block, one MMA step per tile.
+template <int CG, bool DBG, bool WIDE, bool BAND, bool NARROW = false>
 __global__ void __launch_bounds__(384, 1) k_filter_tc(const Args a)
 {
     using SchedT = typename std::conditional<BAND, BandSched<CG>, Sched<CG>>::type;
@@ -284,7 +299,7 @@ __global__ void __launch_bounds__(384, 1) k_filter_tc(const Args a)
     const uint32_t base = (raw + 1023u) & ~1023u;
     const uint32_t k_nc = WIDE ? a.nc : 1u;                               // chunks per row
     const uint32_t k_nabuf = WIDE ? a.n_abuf : 2u;                        // A buffers
-    const uint32_t k_abytes = WIDE ? a.a_bytes : BLOCK_BYTES;             // bytes per A buffer
+    const uint32_t k_abytes = WIDE ? a.a_bytes : NARROW ? NBLOCK_BYTES : BLOCK_BYTES;  // bytes per A buffer
     const uint32_t sA = base, sB = base + k_nabuf * k_abytes, sBar = base + a.data_bytes;
     auto bar_full = [&](uint32_t i) { return sBar + 8 * i; };
     auto bar_pfull = [&](uint32_t i) { return sBar + 8 * (MAXST + i); };
@@ -295,8 +310,11 @@ __global__ void __launch_bounds__(384, 1) k_filter_tc(const Args a)
     // B ring: one stage = one 64-column chunk of a column tile (its hi rows alone with one slice, which gives
     // twice the stages in the same memory); A: all chunks of the row tile, double-buffered over items when it fits
     const uint32_t lg_nst = a.lg_nst, nst_mask = (1u << lg_nst) - 1u, stage_bytes = a.stage_bytes;
-    const uint32_t a_chunk = a.slices == 1 ? SLICE_BYTES : BLOCK_BYTES;  // bytes of one chunk of an A tile in shared memory
-    const uint32_t g_chunk = a.compact ? SLICE_BYTES : BLOCK_BYTES;      // bytes of one chunk of a 128-row block in global memory
+    // bytes of one chunk of an A tile in shared memory, of one slice of a 128-row block, of one chunk of a 128-row
+    // block in global memory
+    const uint32_t a_chunk = NARROW ? NBLOCK_BYTES : a.slices == 1 ? SLICE_BYTES : BLOCK_BYTES;
+    const uint32_t b_slice = NARROW ? NBLOCK_BYTES : SLICE_BYTES;
+    const uint32_t g_chunk = NARROW ? NBLOCK_BYTES : a.compact ? SLICE_BYTES : BLOCK_BYTES;
     const uint64_t gblk = (uint64_t)k_nc * g_chunk;                      // bytes of a 128-row block in global memory
     const uint32_t off_tmem = a.data_bytes + SM::n_bars * 8;
     volatile uint32_t *tmem_slot = reinterpret_cast<volatile uint32_t *>(smem_raw + (base - raw) + off_tmem);
@@ -324,7 +342,7 @@ __global__ void __launch_bounds__(384, 1) k_filter_tc(const Args a)
         SchedT sc;
         sched_init(sc, a, sa, unit, n_units);
         uint32_t I, J0, J1, t = 0, item = 0;
-        const uint32_t nc = k_nc, n_abuf = k_nabuf, a_bytes = k_abytes, slices = a.slices;
+        const uint32_t nc = k_nc, n_abuf = k_nabuf, a_bytes = k_abytes, slices = NARROW ? 1u : a.slices;
         const unsigned char *const HA = a.HA, *const HB = a.HB;
         while (sc.next(I, J0, J1)) {
             const uint32_t ab = n_abuf == 2 ? (item & 1u) : 0u;
@@ -346,8 +364,8 @@ __global__ void __launch_bounds__(384, 1) k_filter_tc(const Args a)
                         } else {
                             // 256 B rows of one CTA: the hi slices of both 128-row blocks, then both lo slices
                             const unsigned char *b0 = HB + (uint64_t)(J * 2) * gblk + (uint64_t)c * g_chunk;
-                            bulk_g2s(dst, b0, SLICE_BYTES, bar_full(st));
-                            bulk_g2s(dst + SLICE_BYTES, b0 + gblk, SLICE_BYTES, bar_full(st));
+                            bulk_g2s(dst, b0, b_slice, bar_full(st));
+                            bulk_g2s(dst + b_slice, b0 + gblk, b_slice, bar_full(st));
                             if (slices != 1) {
                                 bulk_g2s(dst + 2 * SLICE_BYTES, b0 + SLICE_BYTES, SLICE_BYTES, bar_full(st));
                                 bulk_g2s(dst + 3 * SLICE_BYTES, b0 + gblk + SLICE_BYTES, SLICE_BYTES, bar_full(st));
@@ -380,16 +398,21 @@ __global__ void __launch_bounds__(384, 1) k_filter_tc(const Args a)
                         const uint32_t st = t & nst_mask, ph = (t >> lg_nst) & 1u;
                         mbar_wait(bar_full(st), ph, 4);
                         if (CG == 2) mbar_wait(bar_pfull(st), ph, 5);
-                        const uint64_t adesc = make_desc(a_tile + c * a_chunk);
-                        const uint64_t bdesc = make_desc(sB + st * stage_bytes);
+                        const uint64_t adesc = NARROW ? make_desc32(a_tile) : make_desc(a_tile + c * a_chunk);
+                        const uint64_t bdesc = NARROW ? make_desc32(sB + st * stage_bytes) : make_desc(sB + st * stage_bytes);
                         if (c == 0) mbar_wait(bar_tempty(as), ((tile >> 1) & 1u) ^ 1u, 3);
                         fence_after();
                         if (elect_one()) {
-                            // a_hi.b_hi (one slice), then a_lo.b_hi and a_hi.b_lo (two slices)
+                            // a_hi.b_hi (one slice), then a_lo.b_hi and a_hi.b_lo (two slices); narrow: the whole row is
+                            // one K = 16 step
+                            if (NARROW) {
+                                umma_f16<CG>(d_tmem, adesc, bdesc, idesc, 0u);
+                            } else {
 #pragma unroll
-                            for (uint32_t kk = 0; kk < 4; kk++)
-                                umma_f16<CG>(d_tmem, adesc + 2 * kk, bdesc + 2 * kk, idesc, (c | kk) != 0 ? 1u : 0u);
-                            if (n_terms != 1) {
+                                for (uint32_t kk = 0; kk < 4; kk++)
+                                    umma_f16<CG>(d_tmem, adesc + 2 * kk, bdesc + 2 * kk, idesc, (c | kk) != 0 ? 1u : 0u);
+                            }
+                            if (!NARROW && n_terms != 1) {
 #pragma unroll
                                 for (uint32_t kk = 0; kk < 4; kk++)
                                     umma_f16<CG>(d_tmem, adesc + (SLICE_BYTES >> 4) + 2 * kk, bdesc + 2 * kk, idesc, 1u);
@@ -780,10 +803,134 @@ __global__ void __launch_bounds__(256) k_tc_prep(const double *__restrict__ S, u
     }
 }
 
+// ---- projected operands (DESIGN.md "K2-TC", projection) -------------------------------------------
+// Rows of the orthonormalised basis P^ (FP64, zero beyond K), passed by value: every thread reads them as uniform operands.
+struct Basis {
+    double p[PROJ_R][KMAX];
+};
+
+// Second moments about the centre m of the same <= CENTRE_SAMPLE rows k_tc_centre_median reads: one block per entry
+// (i <= j), every thread a fixed stride of the sample, a fixed-order tree in shared memory; no atomics, so every GPU
+// derives the same bits from the same rows. Entries that are not finite, or whose product is not, are skipped.
+__global__ void __launch_bounds__(256) k_tc_cov(const double *__restrict__ S, uint64_t r0, uint64_t r1, uint32_t K,
+                                                const double *__restrict__ centre, double *__restrict__ cov)
+{
+    __shared__ double red[256];
+    uint32_t b = blockIdx.x, i = 0;
+    while (b >= K - i) { b -= K - i; i++; }
+    const uint32_t j = i + b;
+    const uint64_t n = r1 - r0;
+    const uint64_t ns = n < CENTRE_SAMPLE ? n : CENTRE_SAMPLE;
+    double acc = 0.0;
+    for (uint64_t t = threadIdx.x; t < ns; t += blockDim.x) {
+        const uint64_t row = r0 + t * (n / ns);
+        const double p = __dmul_rn(__dsub_rn(S[row * K + i], centre[i]), __dsub_rn(S[row * K + j], centre[j]));
+        if (isfinite(p)) acc = __dadd_rn(acc, p);
+    }
+    red[threadIdx.x] = acc;
+    __syncthreads();
+    for (uint32_t h = blockDim.x / 2; h > 0; h >>= 1) {
+        if (threadIdx.x < h) red[threadIdx.x] = __dadd_rn(red[threadIdx.x], red[threadIdx.x + h]);
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) { cov[i * K + j] = red[0]; cov[j * K + i] = red[0]; }
+}
+
+// y = P^ a', rho = |a' - P^T y| (computed directly: |a'|^2 - |y|^2 cancels when the row lies in the span), FP64, fixed order.
+// a' has K <= KMAX entries, zero beyond.
+__device__ __forceinline__ void proj_row(const Basis &B, const double (&x)[KMAX], double (&y)[PROJ_R], double &rho)
+{
+#pragma unroll
+    for (uint32_t k = 0; k < PROJ_R; k++) {
+        double t = 0.0;
+#pragma unroll
+        for (uint32_t c = 0; c < KMAX; c++) t = fma(B.p[k][c], x[c], t);
+        y[k] = t;
+    }
+    double r2 = 0.0;
+#pragma unroll
+    for (uint32_t c = 0; c < KMAX; c++) {
+        double r = x[c];
+#pragma unroll
+        for (uint32_t k = 0; k < PROJ_R; k++) r = fma(-B.p[k][c], y[k], r);
+        r2 = fma(r, r, r2);
+    }
+    rho = sqrt(r2);
+}
+
+// One thread per row (operand position): the 16-column fp16 image, A [y0 .. y10 rho | x0 x1 P Q] and B [y .. rho | P Q x0 x1],
+// both K-major SWIZZLE_32B. The scale is the centred rows' scale s (k_tc_fix_scale) divided by 8: |y_k|, rho <= |a'| (1 + delta)
+// <= sqrt(60) max_k |a'_k|, so the magnitudes k_tc_prep keeps below 2^12 stay below it here. The fold column carries
+//   h = (|z|^2 (1 - c) - cproj |a'|^2 - T0 (1/2 + 2c) - e0) / 2,   z = (y, rho) scaled, |a'|^2 scaled (NRM s^2),
+// T0 passed with the projection's relative term already in it (tc_prepare). One slice: no lo halves.
+__global__ void __launch_bounds__(128) k_tc_prep_proj(const double *__restrict__ S, uint64_t n, uint64_t r0, uint64_t r1, uint32_t K,
+                                                      const Basis B, const double *__restrict__ NRM,
+                                                      unsigned long long *__restrict__ misc, double T0, double cguard, double cproj,
+                                                      const double *__restrict__ centre, unsigned char *__restrict__ HA,
+                                                      unsigned char *__restrict__ HB)
+{
+    const uint64_t row = r0 + (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (row >= r1) return;
+    const double s = __longlong_as_double((long long)misc[1]) * 0.125;
+    const bool real = row < n;
+    const bool wild = real && !isfinite(NRM[row]);
+    const bool data = real && !wild;
+    double y[PROJ_R], rho = 0.0;
+#pragma unroll
+    for (uint32_t k = 0; k < PROJ_R; k++) y[k] = 0.0;
+    bool too_big = false;
+    double nz = 0.0;
+    if (data) {
+        double x[KMAX];
+#pragma unroll
+        for (uint32_t c = 0; c < KMAX; c++) x[c] = c < K ? __dsub_rn(S[row * K + c], centre[c]) : 0.0;
+        proj_row(B, x, y, rho);
+#pragma unroll
+        for (uint32_t k = 0; k < PROJ_R; k++) {
+            y[k] *= s;
+            too_big |= !(fabs(y[k]) < 4096.0);
+            nz = fma(y[k], y[k], nz);
+        }
+        rho *= s;
+        too_big |= !(rho < 4096.0);
+        nz = fma(rho, rho, nz);
+        if (too_big) {
+            atomicAdd(misc + 2, 1ull);
+            nz = 0.0;
+        }
+    }
+    const double P = 32768.0, Q = 8.0;
+    const double T0s = (T0 * s) * s;
+    const double e0 = (double)K * 0.0078125;
+    const double nfull = data ? (NRM[row] * s) * s : 0.0;
+    const double h = 0.5 * (nz * (1.0 - cguard) - cproj * nfull - T0s * (0.5 + 2.0 * cguard) - e0);
+    double x0, x1;
+    if (!real) { x0 = -65504.0; x1 = 0.0; }                                           // padding row: never a survivor
+    else if (wild || too_big || !(-h <= 32768.0 * P)) { x0 = 65504.0; x1 = 0.0; }     // always a survivor
+    else {
+        x0 = h16z(-h / P);
+        x1 = h16z((-h - P * x0) / Q);
+    }
+    __align__(16) __half va[16], vb[16];
+#pragma unroll
+    for (uint32_t k = 0; k < PROJ_R; k++) va[k] = vb[k] = __double2half(too_big ? 0.0 : h16z(y[k]));
+    va[PROJ_R] = vb[PROJ_R] = __double2half(too_big ? 0.0 : h16z(rho));
+    va[12] = __double2half(x0); va[13] = __double2half(x1); va[14] = __double2half(P); va[15] = __double2half(Q);
+    vb[12] = __double2half(P); vb[13] = __double2half(Q); vb[14] = __double2half(x0); vb[15] = __double2half(x1);
+    const uint32_t r = (uint32_t)(row % ROWS), sw = (r >> 2) & 1u;
+    const uint64_t base = (row / ROWS) * NBLOCK_BYTES + (uint64_t)r * NROW_BYTES;
+    const uint4 *pa = reinterpret_cast<const uint4 *>(va), *pb = reinterpret_cast<const uint4 *>(vb);
+#pragma unroll
+    for (uint32_t c = 0; c < 2; c++) {
+        *reinterpret_cast<uint4 *>(HA + base + 16 * (c ^ sw)) = pa[c];
+        *reinterpret_cast<uint4 *>(HB + base + 16 * (c ^ sw)) = pb[c];
+    }
+}
+
 // ---- survivor-density estimate ---------------------------------------------------------------------
 // PLAN_SAMPLE pseudo-random pairs, one warp each, in FP64: would the pair survive the one-slice filter, the two-slice
-// filter — each with centred and with raw operand copies — and the FP64 DMMA filter? plan[0..4] receive the five
-// counts; the host turns them into survivor estimates and picks the variant BEFORE the first launch (tc_choose),
+// filter — each with centred and with raw operand copies — the FP64 DMMA filter and (proj != 0) the projected filter?
+// plan[0..5] receive the six counts; the host turns them into survivor estimates and picks the variant BEFORE the first launch (tc_choose),
 // instead of finding out by overflowing the queue.
 // Criterion (DESIGN.md "K2-TC"): acc >= 0  <=>  d^2 <= c (|a'|^2 + |b'|^2) + T0 (1 + 4c) + 2 e0 / s^2, a' = a - m.
 constexpr uint32_t PLAN_SAMPLE = 8192;
@@ -794,7 +941,9 @@ __device__ __forceinline__ uint64_t plan_mix(uint64_t z)
     return z ^ (z >> 31);
 }
 __global__ void __launch_bounds__(256) k_tc_plan_sample(const double *__restrict__ S, const double *__restrict__ NRM, uint64_t r0,
-                                                        uint64_t n, uint32_t K, double T0, unsigned long long *__restrict__ misc)
+                                                        uint64_t n, uint32_t K, double T0, unsigned long long *__restrict__ misc,
+                                                        const double *__restrict__ basis, const double *__restrict__ centre, double T0p,
+                                                        double cproj)
 {
     const uint32_t t = blockIdx.x * 8 + (threadIdx.x >> 5);
     const int lane = threadIdx.x & 31;
@@ -816,6 +965,51 @@ __global__ void __launch_bounds__(256) k_tc_plan_sample(const double *__restrict
         ua += __shfl_xor_sync(0xffffffffu, ua, o);
         ub += __shfl_xor_sync(0xffffffffu, ub, o);
     }
+    // projected criterion of k_tc_prep_proj: the warp computes z = (P^ a', |a' - P^T P^ a'|) of both rows
+    // (basis: PROJ_R x KMAX in global memory, nullptr = no projected count)
+    double dz = 0.0, nz = 0.0;
+    const bool proj = basis != nullptr;
+    auto BP = [&](uint32_t k, uint32_t c) { return basis[k * KMAX + c]; };
+    if (proj) {
+        double ya[PROJ_R], yb[PROJ_R];
+#pragma unroll
+        for (uint32_t k = 0; k < PROJ_R; k++) {
+            double ta = 0.0, tb = 0.0;
+            for (uint32_t c = lane; c < K; c += 32) {
+                ta = fma(BP(k, c), S[i * K + c] - centre[c], ta);
+                tb = fma(BP(k, c), S[j * K + c] - centre[c], tb);
+            }
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) {
+                ta += __shfl_xor_sync(0xffffffffu, ta, o);
+                tb += __shfl_xor_sync(0xffffffffu, tb, o);
+            }
+            ya[k] = ta;
+            yb[k] = tb;
+        }
+        double ra = 0.0, rb = 0.0;
+        for (uint32_t c = lane; c < K; c += 32) {
+            double xa = S[i * K + c] - centre[c], xb = S[j * K + c] - centre[c];
+#pragma unroll
+            for (uint32_t k = 0; k < PROJ_R; k++) { xa = fma(-BP(k, c), ya[k], xa); xb = fma(-BP(k, c), yb[k], xb); }
+            ra = fma(xa, xa, ra);
+            rb = fma(xb, xb, rb);
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            ra += __shfl_xor_sync(0xffffffffu, ra, o);
+            rb += __shfl_xor_sync(0xffffffffu, rb, o);
+        }
+        ra = sqrt(ra);
+        rb = sqrt(rb);
+#pragma unroll
+        for (uint32_t k = 0; k < PROJ_R; k++) {
+            dz = fma(ya[k] - yb[k], ya[k] - yb[k], dz);
+            nz = fma(ya[k], ya[k], fma(yb[k], yb[k], nz));
+        }
+        dz = fma(ra - rb, ra - rb, dz);
+        nz = fma(ra, ra, fma(rb, rb, nz));
+    }
     if (lane != 0) return;
     const double s = __longlong_as_double((long long)misc[1]);
     const double nn = NRM[i] + NRM[j];            // centred squared norms (raw ones: ua + ub)
@@ -828,6 +1022,7 @@ __global__ void __launch_bounds__(256) k_tc_plan_sample(const double *__restrict
     if (!(d2 > c1 * (ua + ub) + T0 * (1.0 + 4.0 * c1) + e0)) atomicAdd(plan + 2, 1ull);
     if (!(d2 > c2 * (ua + ub) + T0 * (1.0 + 4.0 * c2) + e0)) atomicAdd(plan + 3, 1ull);
     if (!(d2 > T0 + (4.0 * K + 64.0) * 1.1102230246251565e-16 * 4.0 * (ua + ub))) atomicAdd(plan + 4, 1ull);
+    if (proj && !(dz > c1 * nz + cproj * nn + T0p * (1.0 + 4.0 * c1) + 64.0 * e0)) atomicAdd(plan + 5, 1ull);  // scale s / 8
 }
 
 // ---- norm-band mode -------------------------------------------------------------------------------
@@ -912,6 +1107,176 @@ static int tc_k_headroom(uint32_t K) { return K <= 64 ? 0 : K <= 256 ? 1 : 2; }
 bool tc_supported(const scema_ctx *ctx) { return ctx->K >= 1 && tc_chunks(ctx->K) <= 10; }
 // more than one chunk: hi slices only (the two-slice A tile would not fit next to a B ring)
 bool tc_two_slices_possible(const scema_ctx *ctx) { return tc_chunks(ctx->K) == 1; }
+// the projected filter: rows of one chunk that are wider than its 16 columns
+bool tc_proj_possible(uint32_t K) { return K >= 16 && K <= tc::KMAX; }
+static constexpr double TC_CPROJ = 1.0 / 4294967296.0;       // 2^-32: FP64 rounding of y and rho, relative to |a'|^2
+static constexpr double TC_DELTA_MAX = 1.0 / 4294967296.0;   // largest |P P^T - I|_F the bound accepts
+static constexpr double TC_T0_PROJ = 1.0 + 1.0 / 1073741824.0; // T0 (1 + 2^-30) covers (1 + 2 delta) d^2 on an edge
+
+// cyclic Jacobi on a symmetric m x m matrix H (row-major, destroyed): eigenvalues on its diagonal, eigenvectors the columns of W
+static void jacobi_sym(uint32_t m, std::vector<double> &H, std::vector<double> &W)
+{
+    W.assign((size_t)m * m, 0.0);
+    for (uint32_t i = 0; i < m; i++) W[i * m + i] = 1.0;
+    for (int sweep = 0; sweep < 64; sweep++) {
+        double off = 0.0, dia = 0.0;
+        for (uint32_t p = 0; p < m; p++) {
+            dia += H[p * m + p] * H[p * m + p];
+            for (uint32_t q = p + 1; q < m; q++) off += H[p * m + q] * H[p * m + q];
+        }
+        if (!(off > 1e-32 * dia)) break;   // off-diagonal below 1e-16 of the diagonal: the order of the Ritz values is settled
+        const double small = 1e-18 * std::sqrt(dia);
+        for (uint32_t p = 0; p < m; p++)
+            for (uint32_t q = p + 1; q < m; q++) {
+                const double apq = H[p * m + q];
+                if (!(std::fabs(apq) > small)) continue;
+                const double theta = 0.5 * (H[q * m + q] - H[p * m + p]) / apq;
+                double t = 1.0 / (std::fabs(theta) + std::sqrt(1.0 + theta * theta));
+                if (theta < 0.0) t = -t;
+                const double c = 1.0 / std::sqrt(1.0 + t * t), sn = t * c;
+                for (uint32_t k = 0; k < m; k++) {
+                    const double hkp = H[k * m + p], hkq = H[k * m + q];
+                    H[k * m + p] = c * hkp - sn * hkq;
+                    H[k * m + q] = sn * hkp + c * hkq;
+                }
+                for (uint32_t k = 0; k < m; k++) {
+                    const double hpk = H[p * m + k], hqk = H[q * m + k];
+                    H[p * m + k] = c * hpk - sn * hqk;
+                    H[q * m + k] = sn * hpk + c * hqk;
+                }
+                H[p * m + q] = H[q * m + p] = 0.0;
+                for (uint32_t k = 0; k < m; k++) {
+                    const double wkp = W[k * m + p], wkq = W[k * m + q];
+                    W[k * m + p] = c * wkp - sn * wkq;
+                    W[k * m + q] = sn * wkp + c * wkq;
+                }
+            }
+    }
+}
+
+// modified Gram-Schmidt on the m vectors of length K in V (vector j at V[j * K]); a vector with (almost) nothing left
+// is replaced by the unit vector that keeps the most of itself against the ones before it
+static void mgs(uint32_t m, uint32_t K, std::vector<double> &V)
+{
+    for (uint32_t j = 0; j < m; j++) {
+        double *v = &V[(size_t)j * K];
+        double before = 0.0;
+        for (uint32_t c = 0; c < K; c++) before += v[c] * v[c];
+        for (int attempt = 0;; attempt++) {
+            for (uint32_t i = 0; i < j; i++) {
+                const double *u = &V[(size_t)i * K];
+                double r = 0.0;
+                for (uint32_t c = 0; c < K; c++) r += u[c] * v[c];
+                for (uint32_t c = 0; c < K; c++) v[c] -= r * u[c];
+            }
+            double nn = 0.0;
+            for (uint32_t c = 0; c < K; c++) nn += v[c] * v[c];
+            if (attempt == 0 && nn > 1e-24 * before && nn > 0.0) {
+                const double f = 1.0 / std::sqrt(nn);
+                for (uint32_t c = 0; c < K; c++) v[c] *= f;
+                break;
+            }
+            if (attempt > 0) {
+                const double f = 1.0 / std::sqrt(nn);
+                for (uint32_t c = 0; c < K; c++) v[c] *= f;
+                break;
+            }
+            // degenerate: the unit vector e_b with the largest component outside span(V[0 .. j))
+            uint32_t best = 0;
+            double bres = -1.0;
+            for (uint32_t b = 0; b < K; b++) {
+                double res = 1.0;
+                for (uint32_t i = 0; i < j; i++) res -= V[(size_t)i * K + b] * V[(size_t)i * K + b];
+                if (res > bres) { bres = res; best = b; }
+            }
+            for (uint32_t c = 0; c < K; c++) v[c] = c == best ? 1.0 : 0.0;
+        }
+    }
+}
+
+// Orthonormal basis (PROJ_R rows, basis[k * KMAX + c], zero beyond K) of the leading principal directions of the second
+// moments C [K][K] of the centred sample: block subspace iteration on 16 vectors from a fixed pseudo-random start, then a
+// Rayleigh-Ritz step (Jacobi on the 16 x 16 projection), Ritz vectors by descending Ritz value, each signed so that its
+// largest-magnitude component (first such) is positive, orthonormalised twice by modified Gram-Schmidt. Fixed
+// operation order and no threads: the same C gives the same bits on every host. *delta = |P P^T - I|_F. The filter's
+// bound holds for any basis with a small delta (DESIGN.md "K2-TC"); how well it fits the data only decides how many
+// pairs survive. False when C is not finite, K is outside [16, KMAX] or delta exceeds TC_DELTA_MAX.
+bool tc_basis_from_moments(const double *C, uint32_t K, double *basis, double *delta)
+{
+    constexpr uint32_t M = 16, ITER = 3, R = tc::PROJ_R;
+    *delta = INFINITY;
+    if (!tc_proj_possible(K)) return false;
+    for (uint32_t i = 0; i < K * K; i++)
+        if (!std::isfinite(C[i])) return false;
+    std::vector<double> Q((size_t)M * K), Z((size_t)M * K);
+    uint64_t z = 0x9e3779b97f4a7c15ull;
+    for (auto &q : Q) {
+        z += 0x9e3779b97f4a7c15ull;
+        uint64_t x = z;
+        x = (x ^ (x >> 30)) * 0xbf58476d1ce4e5b9ull;
+        x = (x ^ (x >> 27)) * 0x94d049bb133111ebull;
+        x ^= x >> 31;
+        q = (double)(x >> 11) * 0x1.0p-52 - 1.0;
+    }
+    mgs(M, K, Q);
+    auto mul = [&](const std::vector<double> &in, std::vector<double> &out) {   // out_j = C in_j, column by column (C = C^T)
+        for (uint32_t j = 0; j < M; j++) {
+            double *o = &out[(size_t)j * K];
+            for (uint32_t r = 0; r < K; r++) o[r] = 0.0;
+            for (uint32_t c = 0; c < K; c++) {
+                const double x = in[(size_t)j * K + c];
+                for (uint32_t r = 0; r < K; r++) o[r] += C[c * K + r] * x;
+            }
+        }
+    };
+    for (uint32_t it = 0; it < ITER; it++) {
+        mul(Q, Z);
+        Q.swap(Z);
+        mgs(M, K, Q);
+    }
+    mul(Q, Z);
+    std::vector<double> H((size_t)M * M), W;
+    for (uint32_t a = 0; a < M; a++)
+        for (uint32_t b = a; b < M; b++) {
+            double t = 0.0;
+            for (uint32_t c = 0; c < K; c++) t += Q[(size_t)a * K + c] * Z[(size_t)b * K + c] + Q[(size_t)b * K + c] * Z[(size_t)a * K + c];
+            H[a * M + b] = H[b * M + a] = 0.5 * t;
+        }
+    jacobi_sym(M, H, W);
+    std::vector<uint32_t> ord(M);
+    for (uint32_t i = 0; i < M; i++) ord[i] = i;
+    std::stable_sort(ord.begin(), ord.end(), [&](uint32_t a, uint32_t b) { return H[a * M + a] > H[b * M + b]; });
+    std::vector<double> U((size_t)R * K, 0.0);
+    for (uint32_t k = 0; k < R; k++) {
+        double *u = &U[(size_t)k * K];
+        for (uint32_t j = 0; j < M; j++) {
+            const double w = W[j * M + ord[k]];
+            for (uint32_t c = 0; c < K; c++) u[c] += w * Q[(size_t)j * K + c];
+        }
+    }
+    mgs(R, K, U);
+    mgs(R, K, U);
+    for (uint32_t k = 0; k < R; k++) {
+        double *u = &U[(size_t)k * K];
+        uint32_t big = 0;
+        for (uint32_t c = 1; c < K; c++)
+            if (std::fabs(u[c]) > std::fabs(u[big])) big = c;
+        if (u[big] < 0.0)
+            for (uint32_t c = 0; c < K; c++) u[c] = -u[c];
+    }
+    double f2 = 0.0;
+    for (uint32_t a = 0; a < R; a++)
+        for (uint32_t b = 0; b < R; b++) {
+            double t = 0.0;
+            for (uint32_t c = 0; c < K; c++) t += U[(size_t)a * K + c] * U[(size_t)b * K + c];
+            t -= a == b ? 1.0 : 0.0;
+            f2 += t * t;
+        }
+    *delta = std::sqrt(f2);
+    for (uint32_t k = 0; k < R; k++)
+        for (uint32_t c = 0; c < tc::KMAX; c++) basis[k * tc::KMAX + c] = c < K ? U[(size_t)k * K + c] : 0.0;
+    return *delta <= TC_DELTA_MAX;
+}
 
 // Operand preparation in three steps so that the host-buffer pipeline can run it range by range:
 //   tc_prepare_begin : buffers, threshold constants, guard band of the slice count
@@ -926,6 +1291,7 @@ int tc_prepare_begin(scema_ctx *ctx, double thr, uint32_t slices)
     ctx->tc_valid = false;
     ctx->tc_compact = false;  // [hi | lo] blocks unless a sharded prepare (tc_shard_*) asks for the hi-only layout
     ctx->tc_band = false;  // row order unless tc_prepare sorts by norm afterwards
+    ctx->tc_proj = false;  // 64-column copies unless tc_prepare chooses the projection
     const uint32_t nc = tc_chunks(K);
     if (nc > 1 && slices != 1) return fail(ctx, SCEMA_ERR_INVALID, "tensor-core filter: rows wider than 60 columns run with one slice");
     SCEMA_CUDA(ctx, ctx->d_tc_a.reserve(n_pad * 256 * nc));
@@ -995,6 +1361,17 @@ int tc_fix_scale(scema_ctx *ctx, int headroom)
 int tc_prep_rows(scema_ctx *ctx, uint64_t r0, uint64_t r1)
 {
     if (r1 <= r0) return SCEMA_OK;
+    if (ctx->tc_proj) {
+        tc::Basis B;
+        std::copy(ctx->tc_basis_h, ctx->tc_basis_h + tc::PROJ_R * tc::KMAX, &B.p[0][0]);
+        tc::k_tc_prep_proj<<<(unsigned)((r1 - r0 + 127) / 128), 128, 0, ctx->stream>>>(
+            ctx->d_spline, ctx->n, r0, r1, ctx->K, B, ctx->d_tc_nrm.as<double>(), ctx->d_tc_misc.as<unsigned long long>(),
+            ctx->tc_T0 * TC_T0_PROJ, ctx->tc_cguard, TC_CPROJ, ctx->d_tc_centre.as<double>(), ctx->d_tc_a.as<unsigned char>(),
+            ctx->d_tc_b.as<unsigned char>());
+        ctx->launches++;
+        SCEMA_CUDA(ctx, cudaGetLastError());
+        return SCEMA_OK;
+    }
     tc::k_tc_prep<<<(unsigned)((r1 - r0 + 7) / 8), 256, 0, ctx->stream>>>(
         ctx->d_spline, ctx->n, r0, r1, ctx->K, tc_chunks(ctx->K), ctx->tc_slices, ldexp(1.0, 12 - tc_k_headroom(ctx->K)),
         ctx->d_tc_nrm.as<double>(),
@@ -1007,15 +1384,51 @@ int tc_prep_rows(scema_ctx *ctx, uint64_t r0, uint64_t r1)
     return SCEMA_OK;
 }
 
+// Basis of the projected filter from the centred sample of rows [r0, r1) (the rows k_tc_centre_median read): second
+// moments on the device (k_tc_cov), basis on the host (tc_basis_from_moments) while the device computes the row
+// statistics that were enqueued behind the copy (`then`), basis back to the device for the survivor sample.
+// *ok = false: no usable basis (the 64-column copies stay).
+template <class F>
+static int tc_basis_rows(scema_ctx *ctx, uint64_t r0, uint64_t r1, bool *ok, F then)
+{
+    const uint32_t K = ctx->K;
+    *ok = false;
+    SCEMA_CUDA(ctx, ctx->d_tc_cov.reserve((size_t)K * K * sizeof(double)));
+    SCEMA_CUDA(ctx, ctx->d_tc_basis.reserve(sizeof(ctx->tc_basis_h)));
+    if (!ctx->h_tc_cov) SCEMA_CUDA(ctx, cudaMallocHost(&ctx->h_tc_cov, 60 * 60 * sizeof(double)));
+    tc::k_tc_cov<<<K * (K + 1) / 2, 256, 0, ctx->stream>>>(ctx->d_spline, r0, r1, K, ctx->d_tc_centre.as<double>(), ctx->d_tc_cov.as<double>());
+    ctx->launches++;
+    SCEMA_CUDA(ctx, cudaGetLastError());
+    SCEMA_CUDA(ctx, cudaMemcpyAsync(ctx->h_tc_cov, ctx->d_tc_cov.p, (size_t)K * K * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    cudaEvent_t ev;
+    SCEMA_CUDA(ctx, cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+    cudaError_t e = cudaEventRecord(ev, ctx->stream);
+    int rc = e == cudaSuccess ? then() : SCEMA_OK;
+    if (e == cudaSuccess) e = cudaEventSynchronize(ev);
+    cudaEventDestroy(ev);
+    if (e != cudaSuccess) return fail(ctx, SCEMA_ERR_CUDA, std::string("tc basis: ") + cudaGetErrorString(e));
+    if (rc) return rc;
+    double delta = 0.0;
+    *ok = tc_basis_from_moments(ctx->h_tc_cov, K, ctx->tc_basis_h, &delta);
+    if (*ok)
+        SCEMA_CUDA(ctx, cudaMemcpyAsync(ctx->d_tc_basis.p, ctx->tc_basis_h, sizeof(ctx->tc_basis_h), cudaMemcpyHostToDevice, ctx->stream));
+    return SCEMA_OK;
+}
+
+int tc_basis_range(scema_ctx *ctx, uint64_t r0, uint64_t r1, bool *ok)
+{
+    return tc_basis_rows(ctx, r0, r1, ok, [] { return SCEMA_OK; });
+}
+
 // Which filter should evaluate `pairs` pairs of rows of K columns, given how many of `sample` random pairs would survive
-// the one-slice / two-slice tcgen05 filter with centred copies (counts[0], [1]), with raw copies (counts[2], [3]) and the
-// DMMA filter (counts[4])? Cost model in seconds on one B200 (measured rates, DESIGN.md section 6): filter time + exact
+// the one-slice / two-slice tcgen05 filter with centred copies (counts[0], [1]), with raw copies (counts[2], [3]), the
+// DMMA filter (counts[4]) and (proj_ok) the projected filter (counts[5])? Cost model in seconds on one B200 (measured rates, DESIGN.md section 6): filter time + exact
 // recompute of the estimated survivors; a queue that would not fit `mem_budget` bytes rules an option out; raw copies
 // must beat the centred ones by 20 % to be taken. Fewer than four hits in the sample are noise as far as SIZING a queue
 // goes (one hit in 8192 stands for 6e7 survivors at 1M rows). Pure host logic (scema_tc_choose: CPU tests).
-//   -> choice: 1 / 2 = tcgen05 with that many slices, 0 = SCEMA_PAIRS_DMMA, -1 = SCEMA_PAIRS_EXACT; centred: which copies;
-//      est_survivors: queue entries to expect for the choice.
-void tc_choose(uint64_t pairs, uint32_t K, const uint64_t counts[5], uint64_t sample, uint64_t mem_budget, bool tc_ok,
+//   -> choice: 1 / 2 = tcgen05 with that many slices, 3 = the projected tcgen05 filter (centred), 0 = SCEMA_PAIRS_DMMA,
+//      -1 = SCEMA_PAIRS_EXACT; centred: which copies; est_survivors: queue entries to expect for the choice.
+void tc_choose(uint64_t pairs, uint32_t K, const uint64_t counts[6], uint64_t sample, uint64_t mem_budget, bool tc_ok, bool proj_ok,
                int *choice, int *centred, uint64_t *est_survivors)
 {
     const uint32_t nc = tc_chunks(K);
@@ -1037,11 +1450,13 @@ void tc_choose(uint64_t pairs, uint32_t K, const uint64_t counts[5], uint64_t sa
     if (tc_ok) consider(1, 0, R1, counts[2]);
     if (tc_ok && nc == 1) consider(2, 1, R2, counts[1]);
     if (tc_ok) consider(1, 1, R1, counts[0]);
+    if (tc_ok && proj_ok && nc == 1 && tc_proj_possible(K)) consider(3, 1, RATE_TCP, counts[5]);
 }
 
 // Builds (or reuses) the fp16 operand copies for the current spline matrix and threshold.
-// slices: 1 or 2 pins the number of fp16 slices; 0 = decide from a sample of the pairs (k_tc_plan_sample, tc_choose):
-// *choice then returns what was decided (1 / 2 slices, 0: the caller should take SCEMA_PAIRS_DMMA, -1: SCEMA_PAIRS_EXACT —
+// slices: 1 or 2 pins the number of fp16 slices, 3 the projected filter (one slice of 16 columns; 1 slice where the rows
+// do not allow it); 0 = decide from a sample of the pairs (k_tc_plan_sample, tc_choose):
+// *choice then returns what was decided (1 / 2 slices, 3: projected, 0: the caller should take SCEMA_PAIRS_DMMA, -1: SCEMA_PAIRS_EXACT —
 // no operand copies are built in those two cases) and *est_survivors the estimate behind it. `pairs` = pairs this
 // context will evaluate (its shard). want_band: sort the rows by norm first (operand copies in sorted order,
 // ctx->d_tc_perm maps a position back to its row) so that the launch can restrict itself to the band of tiles the
@@ -1054,34 +1469,43 @@ int tc_prepare(scema_ctx *ctx, double thr, uint32_t slices, bool want_band, uint
     if (choice) *choice = (int)slices;
     if (est_survivors) *est_survivors = 0;
     if (ctx->tc_for_version == ctx->spline_version && ctx->tc_thr == thr && ctx->tc_n == n && ctx->tc_K == ctx->K &&
-        (slices == 0 || ctx->tc_slices == slices) && ctx->tc_valid && ctx->tc_band_wanted == want_band) {
-        if (choice) *choice = (int)ctx->tc_slices;   // the same rows and threshold: the earlier decision stands
+        (slices == 0 || (slices == 3 ? ctx->tc_proj : !ctx->tc_proj && ctx->tc_slices == slices)) && ctx->tc_valid &&
+        ctx->tc_band_wanted == want_band) {
+        if (choice) *choice = ctx->tc_proj ? 3 : (int)ctx->tc_slices;   // the same rows and threshold: the earlier decision stands
         return SCEMA_OK;
     }
     const bool two_ok = tc_two_slices_possible(ctx);
+    // the projection needs rows of 16 .. 60 columns and row order (the norm-band mode sorts the 64-column copies)
+    bool proj_ok = (slices == 0 || slices == 3) && !want_band && tc_proj_possible(ctx->K) && n >= 2;
     int rc = wait_rows(ctx);   // a full prepare reads every row
     if (rc) return rc;
-    rc = tc_prepare_begin(ctx, thr, slices ? slices : 1);
+    rc = tc_prepare_begin(ctx, thr, slices == 0 || slices == 3 ? 1 : slices);
     ctx->tc_band = false;
     ctx->tc_band_wanted = want_band;
     if (!rc) rc = tc_centre_rows(ctx, 0, n);
-    if (!rc) rc = tc_stats_rows(ctx, 0, n, true);
-    if (!rc) rc = tc_fix_scale(ctx, 0);
+    auto stats = [&]() {
+        int r = tc_stats_rows(ctx, 0, n, true);
+        return r ? r : tc_fix_scale(ctx, 0);
+    };
+    if (!rc) rc = proj_ok ? tc_basis_rows(ctx, 0, n, &proj_ok, stats) : stats();
     if (rc) return rc;
+    if (slices == 3) slices = 1;   // pinned projection: one slice, 16 columns (64 where the rows do not allow it)
+    else if (slices != 0) proj_ok = false;
     unsigned long long misc[8] = {};
     bool have_misc = false;
     if (slices == 0 && n >= 2) {
-        uint64_t counts[5];
-        rc = tc_plan_rows(ctx, n, counts);
+        uint64_t counts[6];
+        rc = tc_plan_rows(ctx, n, counts, proj_ok);
         if (rc) return rc;
         int ch = 1, centred = 1;
         uint64_t est = 0;
-        tc_choose(pairs, ctx->K, counts, tc::PLAN_SAMPLE, (uint64_t)ctx->mem_budget, true, &ch, &centred, &est);
+        tc_choose(pairs, ctx->K, counts, tc::PLAN_SAMPLE, (uint64_t)ctx->mem_budget, true, proj_ok, &ch, &centred, &est);
         if (ch == 2 && !two_ok) ch = 1;
         if (choice) *choice = ch;
         if (est_survivors) *est_survivors = est;
         if (ch <= 0) return SCEMA_OK;  // the caller takes the DMMA / the filter-free kernel
-        slices = (uint32_t)ch;
+        proj_ok = ch == 3;
+        slices = ch == 3 ? 1u : (uint32_t)ch;
         ctx->tc_slices = slices;
         ctx->tc_cguard = slices == 1 ? 0.001953125 : 0.0001220703125;
         if (!centred) {
@@ -1094,7 +1518,10 @@ int tc_prepare(scema_ctx *ctx, double thr, uint32_t slices, bool want_band, uint
         }
     } else if (slices == 0) {
         slices = 1;
+        proj_ok = false;
     }
+    ctx->tc_proj = proj_ok;
+    if (proj_ok && choice) *choice = 3;
     if (want_band && tc_chunks(ctx->K) == 1) {
         if (!have_misc) {
             SCEMA_CUDA(ctx, cudaMemcpyAsync(misc, ctx->d_tc_misc.p, sizeof(misc), cudaMemcpyDeviceToHost, ctx->stream));
@@ -1126,19 +1553,21 @@ int tc_prepare(scema_ctx *ctx, double thr, uint32_t slices, bool want_band, uint
 
 // Survivor-density sample over the rows [0, r1) (all rows; host-buffer pipeline: the first range, after its statistics
 // and scale). counts = pairs of tc::PLAN_SAMPLE that would survive one slice / two slices with centred copies, the same
-// with raw copies, the DMMA filter. One host synchronisation.
-int tc_plan_rows(scema_ctx *ctx, uint64_t r1, uint64_t counts[5])
+// with raw copies, the DMMA filter, the projected filter (proj: with the basis tc_basis_rows left on the device; 0
+// otherwise). One host synchronisation.
+int tc_plan_rows(scema_ctx *ctx, uint64_t r1, uint64_t counts[6], bool proj)
 {
-    for (int i = 0; i < 5; i++) counts[i] = 0;
+    for (int i = 0; i < 6; i++) counts[i] = 0;
     if (r1 < 2) return SCEMA_OK;
     unsigned long long *d_plan = ctx->d_tc_misc.as<unsigned long long>() + tc::PLAN_WORD, plan[8];
     SCEMA_CUDA(ctx, cudaMemsetAsync(d_plan, 0, 8 * sizeof(unsigned long long), ctx->stream));
-    tc::k_tc_plan_sample<<<tc::PLAN_SAMPLE / 8, 256, 0, ctx->stream>>>(ctx->d_spline, ctx->d_tc_nrm.as<double>(), 0, r1, ctx->K, ctx->tc_T0,
-                                                                     ctx->d_tc_misc.as<unsigned long long>());
+    tc::k_tc_plan_sample<<<tc::PLAN_SAMPLE / 8, 256, 0, ctx->stream>>>(
+        ctx->d_spline, ctx->d_tc_nrm.as<double>(), 0, r1, ctx->K, ctx->tc_T0, ctx->d_tc_misc.as<unsigned long long>(),
+        proj ? ctx->d_tc_basis.as<double>() : nullptr, ctx->d_tc_centre.as<double>(), ctx->tc_T0 * TC_T0_PROJ, TC_CPROJ);
     ctx->launches++;
     SCEMA_CUDA(ctx, cudaMemcpyAsync(plan, d_plan, sizeof(plan), cudaMemcpyDeviceToHost, ctx->stream));
     SCEMA_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    for (int i = 0; i < 5; i++) ctx->tc_plan_counts[i] = counts[i] = plan[i];
+    for (int i = 0; i < 6; i++) ctx->tc_plan_counts[i] = counts[i] = plan[i];
     return SCEMA_OK;
 }
 uint32_t tc_plan_sample_size() { return tc::PLAN_SAMPLE; }
@@ -1212,7 +1641,8 @@ int tc_shard_stats(scema_ctx *ctx, const double *centre_dev, const unsigned long
     if (rc) return rc;
     if (r1 - r0 >= 2) {
         tc::k_tc_plan_sample<<<tc::PLAN_SAMPLE / 8, 256, 0, ctx->stream>>>(ctx->d_spline, ctx->d_tc_nrm.as<double>(), r0, r1 - r0, ctx->K,
-                                                                         ctx->tc_T0, ctx->d_tc_misc.as<unsigned long long>());
+                                                                         ctx->tc_T0, ctx->d_tc_misc.as<unsigned long long>(), nullptr,
+                                                                         nullptr, 0.0, 0.0);
         ctx->launches++;
         SCEMA_CUDA(ctx, cudaGetLastError());
     }
@@ -1262,12 +1692,14 @@ int tc_shard_finish(scema_ctx *ctx, const unsigned long long *packets_dev, uint3
 int tc_shard_check(scema_ctx *ctx, int *choice, uint64_t *est_survivors)
 {
     if (!ctx->plan_pending || !ctx->h_plan) return fail(ctx, SCEMA_ERR_STATE, "tc_shard_check: no sharded prepare to check");
-    uint64_t counts[5];
-    for (int i = 0; i < 5; i++) ctx->tc_plan_counts[i] = counts[i] = ctx->h_plan[i];
+    // the sharded prepare all-gathers 64-column images: the projected filter is never a candidate here
+    uint64_t counts[6];
+    for (int i = 0; i < 6; i++) ctx->tc_plan_counts[i] = counts[i] = i < 5 ? ctx->h_plan[i] : 0;
     ctx->plan_pending = false;
     int ch = 1, centred = 1;
     uint64_t est = 0;
-    tc_choose(ctx->plan_pairs, ctx->K, counts, (uint64_t)tc::PLAN_SAMPLE * ctx->plan_shards, (uint64_t)ctx->mem_budget, true, &ch, &centred, &est);
+    tc_choose(ctx->plan_pairs, ctx->K, counts, (uint64_t)tc::PLAN_SAMPLE * ctx->plan_shards, (uint64_t)ctx->mem_budget, true, false, &ch,
+              &centred, &est);
     *choice = (ch == 1 && centred) ? 1 : (ch == 1 ? 3 : ch);   // 3: one slice but raw copies -> ordinary path
     if (est_survivors) *est_survivors = est;
     return SCEMA_OK;
@@ -1287,10 +1719,10 @@ int tc_shard_commit(scema_ctx *ctx, void *rows_ready_event)
     return SCEMA_OK;
 }
 
-template <int CG, bool DBG, bool WIDE, bool BAND>
+template <int CG, bool DBG, bool WIDE, bool BAND, bool NARROW = false>
 static int tc_launch_t(scema_ctx *ctx, const tc::Args &a, uint64_t items)
 {
-    auto kern = tc::k_filter_tc<CG, DBG, WIDE, BAND>;
+    auto kern = tc::k_filter_tc<CG, DBG, WIDE, BAND, NARROW>;
     const size_t smem = (size_t)a.data_bytes + tc::Smem<CG>::tail;
     if (smem > ctx->smem_optin) return fail(ctx, SCEMA_ERR_CUDA, "tensor-core filter: shared memory exceeds device limit");
     SCEMA_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -1389,6 +1821,16 @@ int tc_launch(scema_ctx *ctx, uint32_t I0, uint32_t I1, uint32_t C0, uint32_t C1
     // items of this shard (upper bound is enough to size the grid)
     const uint64_t n_strips = (cols + a.strip_len - 1) / a.strip_len + 1;
     const uint64_t items = std::max<uint64_t>(1, rows * (2 / cg) * n_strips / std::max<uint32_t>(n_shards, 1));
+    if (ctx->tc_proj) {
+        // projected operands: 4 KB A buffers, a 16-deep ring of B stages (one column tile each: 4 KB per CTA of a pair)
+        a.a_bytes = tc::NBLOCK_BYTES;
+        a.n_abuf = 2;
+        a.lg_nst = 4;
+        a.stage_bytes = (tc::COLT / (uint32_t)cg) * tc::NROW_BYTES;
+        a.data_bytes = a.n_abuf * a.a_bytes + (a.stage_bytes << a.lg_nst);
+        if (cg == 1) return dbg ? tc_launch_t<1, true, false, false, true>(ctx, a, items) : tc_launch_t<1, false, false, false, true>(ctx, a, items);
+        return dbg ? tc_launch_t<2, true, false, false, true>(ctx, a, items) : tc_launch_t<2, false, false, false, true>(ctx, a, items);
+    }
     if (!tc_smem_plan(a.nc, a.slices, (uint32_t)cg, &a.a_bytes, &a.n_abuf, &a.lg_nst, &a.stage_bytes, &a.data_bytes))
         return fail(ctx, SCEMA_ERR_INVALID, "tensor-core filter: row tile does not fit shared memory");
     if (ctx->tc_band && !dbg && a.nc == 1) {
@@ -1418,18 +1860,22 @@ int tc_launch(scema_ctx *ctx, uint32_t I0, uint32_t I1, uint32_t C0, uint32_t C1
 // Debug / validation entry (scema_tc_debug): runs the instrumented kernel over the whole pair matrix
 // and returns every accumulator (acc_host[row * ld + col], ld >= n_pad) and the operand copies, so a
 // test can redo the sliced contraction in FP64 and check the layout, the fold columns and the
-// accumulation-error model against the hardware.
+// accumulation-error model against the hardware. slices = 3: the projected filter (operand copies of
+// n_pad x 32 bytes).
 int tc_debug_run(scema_ctx *ctx, double thr, uint32_t slices, float *acc_host, uint64_t ld, unsigned char *ha_host,
                  unsigned char *hb_host)
 {
-    if (slices != 1 && slices != 2) return fail(ctx, SCEMA_ERR_INVALID, "tc_debug: slices must be 1 or 2");
+    if (slices < 1 || slices > 3) return fail(ctx, SCEMA_ERR_INVALID, "tc_debug: slices must be 1, 2 or 3");
     if (!ctx->have_spline) return fail(ctx, SCEMA_ERR_STATE, "Spline is not up to date.");
     if (!tc_supported(ctx) || !tc_two_slices_possible(ctx)) return fail(ctx, SCEMA_ERR_INVALID, "tc_debug needs 1 <= K <= 60");
+    if (slices == 3 && !tc_proj_possible(ctx->K)) return fail(ctx, SCEMA_ERR_INVALID, "tc_debug: the projected filter needs 16 <= K <= 60");
     const uint64_t n_pad = (ctx->n + tc::COLT - 1) / tc::COLT * tc::COLT;
     if (ld < n_pad) return fail(ctx, SCEMA_ERR_INVALID, "tc_debug: ld < padded n");
     if (n_pad > 8192) return fail(ctx, SCEMA_ERR_INVALID, "tc_debug: at most 8192 rows");
     int rc = tc_prepare(ctx, thr, slices, false, 0, nullptr, nullptr);
     if (rc) return rc;
+    if (slices == 3 && !ctx->tc_proj) return fail(ctx, SCEMA_ERR_STATE, "tc_debug: no usable basis for the projected filter");
+    const uint64_t img = n_pad * (ctx->tc_proj ? tc::NROW_BYTES : 256u);
     SCEMA_CUDA(ctx, ctx->d_counters.reserve(8 * sizeof(uint64_t)));
     SCEMA_CUDA(ctx, cudaMemsetAsync(ctx->d_counters.p, 0, 8 * sizeof(uint64_t), ctx->stream));
     if (ctx->cand_cap == 0) ctx->cand_cap = 1ull << 20;
@@ -1443,8 +1889,8 @@ int tc_debug_run(scema_ctx *ctx, double thr, uint32_t slices, float *acc_host, u
     cudaError_t e = cudaStreamSynchronize(ctx->stream);
     if (e == cudaSuccess && acc_host)
         e = cudaMemcpy2D(acc_host, ld * sizeof(float), dbg.p, n_pad * sizeof(float), n_pad * sizeof(float), n_pad, cudaMemcpyDeviceToHost);
-    if (e == cudaSuccess && ha_host) e = cudaMemcpy(ha_host, ctx->d_tc_a.p, n_pad * 256, cudaMemcpyDeviceToHost);
-    if (e == cudaSuccess && hb_host) e = cudaMemcpy(hb_host, ctx->d_tc_b.p, n_pad * 256, cudaMemcpyDeviceToHost);
+    if (e == cudaSuccess && ha_host) e = cudaMemcpy(ha_host, ctx->d_tc_a.p, img, cudaMemcpyDeviceToHost);
+    if (e == cudaSuccess && hb_host) e = cudaMemcpy(hb_host, ctx->d_tc_b.p, img, cudaMemcpyDeviceToHost);
     dbg.release();
     if (e != cudaSuccess) return fail(ctx, SCEMA_ERR_CUDA, std::string("tc_debug: ") + cudaGetErrorString(e));
     return SCEMA_OK;
