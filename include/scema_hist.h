@@ -152,6 +152,26 @@ int scema_get_degrees(scema_ctx *ctx, uint32_t *degree_host);
  * what scema_compare(+inf, SCEMA_PAIRS_EXACT) returns. Host arrays [n]; either may be NULL. */
 int scema_nearest(scema_ctx *ctx, uint32_t *nearest_id_host, double *nearest_diff_host);
 
+/* k nearest neighbours of every history of the current spline matrix, exact (1 <= k <= 32, otherwise SCEMA_ERR_INVALID;
+ * SCEMA_ERR_STATE without a spline matrix). Row i's k slots are [i*k, i*k + k) of both host arrays (either may be NULL):
+ * index_host the batch indices (not IDs) of the partners, diff_host compare_L2_norm(i, j) with the reference's bits.
+ * Slots in order of (diff, ids[j], j) ascending — the reference's tie-break to the lower ID, then the index, because IDs
+ * may repeat after scema_select_rows. A history is never its own neighbour; partners at distance NaN are skipped (as in
+ * scema_nearest), partners at +inf are listed; unused slots are {UINT32_MAX, +inf} (k > n - 1, rows with a NaN, n <= 1).
+ * With k = 1, ids[index[i]] and the diff bits are what scema_nearest returns.
+ * variant picks the filter of the rounds (SCEMA_PAIRS_TC with its fallbacks, _DMMA, _FMA): a thresholded compare at a radius
+ * from a distance sample closes every row with at least k partners below it, later rounds repeat it for the open rows at a
+ * larger radius, and the rows left over (all rows with SCEMA_PAIRS_EXACT or a small batch, and whenever a round would list
+ * more than O(n k) edges) are evaluated against every history by an exact top-k kernel. The result is bit-identical for
+ * every variant; memory is O(n k). The last compare's edges, degrees, timings, counters, audit and operand caches of this
+ * context are left as they were, also when the call fails. */
+int scema_knn(scema_ctx *ctx, uint32_t k, int variant, uint32_t *index_host, double *diff_host);
+/* The last scema_knn: counts = {filter rounds run, rows finished in round 1, rows finished in later filter rounds, rows
+ * finished by the exact kernel, pairs the exact kernel evaluated, filter survivors over all rounds, edges below the radius
+ * over all rounds, filter variant of the last round (SCEMA_PAIRS_EXACT when none ran)}; radii = the radius of each round
+ * (0 for rounds not run). Either pointer may be NULL. */
+int scema_knn_last_stats(scema_ctx *ctx, uint64_t counts[8], double radii[8]);
+
 /* One call for a host caller: set_histories + resample + compare. With SCEMA_PAIRS_TC, 6 * spline_points <= 60
  * and a large batch (>= 65536 histories; SCEMA_PIPELINE=0 disables, SCEMA_PIPELINE_MIN_N moves the limit) the three
  * steps are pipelined range by range behind the host->device copy of the raw steps: range c is resampled and compared

@@ -57,6 +57,8 @@ def lib():
         "scema_get_degrees": (i32, [vp, vp]),
         "scema_cluster": (i32, [vp, vp, vp, vp, u64, u32, dbl, i32, P(u64)]),
         "scema_nearest": (i32, [vp, vp, vp]),
+        "scema_knn": (i32, [vp, u32, i32, vp, vp]),
+        "scema_knn_last_stats": (i32, [vp, vp, vp]),
         "scema_write_similar_hist": (i32, [vp, C.c_char_p]),
         "scema_reduce_edges": (i32, [vp, u32, vp, P(u64), P(u64)]),
         "scema_reduce_calls": (i32, [vp, vp, u64, u32, vp, P(u64), P(u64)]),
@@ -121,7 +123,7 @@ EXPORTED = (
     "scema_create scema_destroy scema_last_error scema_version scema_stream scema_set_histories scema_resample "
     "scema_store_reset scema_store_append scema_store_info scema_store_resample scema_select_rows "
     "scema_set_spline scema_get_spline scema_spline_info scema_compare scema_compare_stream scema_get_edges scema_edges_device "
-    "scema_get_degrees scema_cluster scema_nearest scema_write_similar_hist scema_reduce_edges scema_reduce_calls scema_reduce_dir "
+    "scema_get_degrees scema_cluster scema_nearest scema_knn scema_knn_last_stats scema_write_similar_hist scema_reduce_edges scema_reduce_calls scema_reduce_dir "
     "scema_last_timings scema_last_counters scema_kernel_launches scema_last_audit scema_fp64_peak scema_k1_tune scema_tc_debug scema_tc_plan scema_tc_shard_begin scema_tc_shard_stats scema_tc_shard_finish scema_tc_shard_check scema_tc_shard_commit scema_tc_centre scema_tc_last_plan scema_tc_choose scema_tc_choose_projected scema_tc_basis scema_tc_last_projection scema_pipeline_plan scema_synth_offsets "
     "scema_multi_create scema_multi_destroy scema_multi_last_error scema_multi_devices scema_multi_context scema_multi_cluster "
     "scema_multi_compare_rows scema_multi_shard_edges scema_multi_last_ms "
@@ -418,6 +420,26 @@ class HistCluster:
         d = np.empty(n, dtype=np.float64)
         self._ck(self._L.scema_nearest(self._h, _ptr(ids), _ptr(d)))
         return ids, d
+
+    def knn(self, k, variant=PAIRS_TC):
+        """Exact k nearest neighbours of every history: (index [n, k] uint32, diff [n, k] float64), slots in order of
+        (diff, ID, index); empty slots are (0xffffffff, inf)."""
+        n, _, _ = self.spline_info()
+        kk = max(int(k), 0)
+        index = np.empty((n, kk), dtype=np.uint32)
+        diff = np.empty((n, kk), dtype=np.float64)
+        self._ck(self._L.scema_knn(self._h, int(k) & 0xffffffff, int(variant), _ptr(index), _ptr(diff)))
+        return index, diff
+
+    def knn_last_stats(self):
+        """What the last knn did: filter rounds, rows finished per stage, exact pairs, survivors, edges, last filter
+        variant and the radius of every round."""
+        c = (C.c_uint64 * 8)()
+        r = (C.c_double * 8)()
+        self._ck(self._L.scema_knn_last_stats(self._h, c, r))
+        return {"rounds": int(c[0]), "rows_round1": int(c[1]), "rows_later_rounds": int(c[2]), "rows_exact": int(c[3]),
+                "exact_pairs": int(c[4]), "survivors": int(c[5]), "edges": int(c[6]), "variant": int(c[7]),
+                "radii": [float(x) for x in r][:int(c[0])]}
 
     def cluster(self, steps, offsets, ids, spline_points, threshold, variant=PAIRS_TC):
         steps = np.ascontiguousarray(steps, dtype=np.float64)

@@ -67,6 +67,8 @@ void scema_destroy(scema_ctx *c)
     for (int i = 0; i < 2 * SCEMA_T_COUNT; i++) if (c->ev[i]) cudaEventDestroy(c->ev[i]);
     for (cudaEvent_t e : c->copy_events) cudaEventDestroy(e);
     if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
+    if (c->knn_child) scema_destroy(c->knn_child);
+    for (scema::DevBuf &b : c->knn_buf) b.release();
     if (c->own_stream) cudaStreamDestroy(c->stream);
     delete c;
 }
@@ -334,6 +336,23 @@ int scema_nearest(scema_ctx *c, uint32_t *nearest_id_host, double *nearest_diff_
     int rc = enter(c);
     if (rc) return rc;
     return nearest_run(c, nearest_id_host, nearest_diff_host);
+}
+
+int scema_knn(scema_ctx *c, uint32_t k, int variant, uint32_t *index_host, double *diff_host)
+{
+    int rc = enter(c);
+    if (rc) return rc;
+    return knn_run(c, k, variant, index_host, diff_host);
+}
+
+int scema_knn_last_stats(scema_ctx *c, uint64_t counts[8], double radii[8])
+{
+    if (!c) return SCEMA_ERR_INVALID;
+    for (int i = 0; i < 8; i++) {
+        if (counts) counts[i] = c->knn_counts[i];
+        if (radii) radii[i] = c->knn_radii[i];
+    }
+    return SCEMA_OK;
 }
 
 int scema_cluster(scema_ctx *c, const double *steps, const uint64_t *offsets, const uint32_t *ids, uint64_t n,

@@ -165,6 +165,13 @@ struct scema_ctx {
     float acc_ms[SCEMA_T_COUNT] = {};  // phases already folded in by earlier chunks of a streamed compare
     uint64_t counters[8] = {};
     uint64_t audit_edges = 0, audit_missing = 0;  // last SCEMA_AUDIT run: sampled pairs that are reference edges / of those, missing from the list
+
+    // ---- scema_knn (knn.cu): the filter rounds run on a private child context (on the same device and stream) so that
+    //      this context's compare results stay as they are; scratch buffers and the stats of the last call
+    scema_ctx *knn_child = nullptr;
+    scema::DevBuf knn_buf[16];
+    uint64_t knn_counts[8] = {};
+    double knn_radii[8] = {};
 };
 
 namespace scema {
@@ -177,6 +184,18 @@ namespace scema {
             return e__ == cudaErrorMemoryAllocation ? SCEMA_ERR_NOMEM : SCEMA_ERR_CUDA;         \
         }                                                                                       \
     } while (0)
+
+// exact pair distance: compare_L2_norm, strain2spline.h:476-483, operation for operation
+__device__ __forceinline__ double exact_l2(const double *__restrict__ a, const double *__restrict__ b, uint32_t K)
+{
+    double sum = 0.0;
+#pragma unroll 4
+    for (uint32_t k = 0; k < K; k++) {
+        double diff = __dsub_rn(__ldg(a + k), __ldg(b + k));
+        sum = __dadd_rn(sum, __dmul_rn(diff, diff));
+    }
+    return __dsqrt_rn(sum);
+}
 
 // IDs of the current spline rows, filled on first use when they are the default 0 .. n-1
 inline const std::vector<uint32_t> &ids_of(scema_ctx *c)
@@ -214,6 +233,7 @@ int compare_stream_run(scema_ctx *ctx, double thr, int variant, uint32_t shard, 
                        scema_edge_sink sink, void *user, uint64_t *n_total);
 int fp64_peak_run(scema_ctx *ctx, double out[2]);
 int nearest_run(scema_ctx *ctx, uint32_t *nearest_id_host, double *nearest_diff_host);
+int compare_prefix_run(scema_ctx *ctx, double thr, int *variant, uint32_t p1);
 int edges_adopt(scema_ctx *ctx, const uint64_t *d_keys, const double *d_vals, uint64_t total);
 bool pipeline_wanted(uint64_t n);
 void pipeline_bounds(uint64_t n, std::vector<uint64_t> &bounds);
@@ -248,6 +268,8 @@ int tc_launch(scema_ctx *ctx, uint32_t I0, uint32_t I1, uint32_t C0, uint32_t C1
               unsigned long long *cand_count, float *dbg, uint64_t dbg_ld);
 int tc_debug_run(scema_ctx *ctx, double thr, uint32_t slices, float *acc_host, uint64_t ld, unsigned char *ha_host,
                  unsigned char *hb_host);
+// knn.cu
+int knn_run(scema_ctx *ctx, uint32_t k, int variant, uint32_t *index_host, double *diff_host);
 // host_io.cc
 int write_similar_hist(scema_ctx *ctx, const char *pattern);
 int reduce_graph_calls(const uint32_t *eu, const uint32_t *ev, uint64_t n_calls, uint32_t num_gps,
