@@ -180,8 +180,11 @@ int scema_knn_last_stats(scema_ctx *ctx, uint64_t counts[8], double radii[8]);
 int scema_cluster(scema_ctx *ctx, const double *steps, const uint64_t *offsets, const uint32_t *ids,
                   uint64_t n, uint32_t spline_points, double threshold, int variant, uint64_t *n_edges);
 
-/* ---- sharded prepare of the tcgen05 filter (one context per GPU, each owning the rows [row0, row1), row0 a multiple of
- *      128, of a spline matrix whose full-size buffer has been installed with scema_set_spline): every GPU builds the fp16
+/* ---- sharded prepare of the tcgen05 filter (one context per GPU, each owning the rows [row0, row1) of a spline matrix
+ *      whose full-size buffer has been installed with scema_set_spline; the shares cover [0, n) without overlap, row0 is a
+ *      multiple of 128 and row1 a multiple of 128 or n — except for an EMPTY share, row0 == row1 at any row <= n, which a
+ *      GPU past the end of a split into equal shares gets: it takes part in every step, contributes no rows, no sample and
+ *      no image): every GPU builds the fp16
  *      operand image of its own rows only and the caller all-gathers the images (128 bytes per row and 64-column chunk)
  *      instead of waiting for the FP64 rows of everybody (8 K bytes per row), which only the exact recompute needs:
  *        scema_tc_shard_begin   -> *centre_dev: K doubles on the device (centre candidate of the own rows); all-gather them
@@ -189,14 +192,18 @@ int scema_cluster(scema_ctx *ctx, const double *steps, const uint64_t *offsets, 
  *        scema_tc_shard_stats   -> *packet_dev: *packet_words 8-byte words (norm statistics and the survivor-density sample
  *                                  of the own rows); all-gather the packets of all n_shards GPUs and pass them to
  *        scema_tc_shard_finish  (optimistic = 0) -> *choice: 1 = one fp16 slice with centred copies: the own rows' image now sits at
- *                                  *image_dev + row0 * *image_bytes_per_row (hi-only layout); all-gather the images in
- *                                  place, then scema_tc_shard_commit. Any other value (2: two slices, 3: raw copies,
+ *                                  *image_dev + row0 * *image_bytes_per_row (hi-only layout; the share that ends at n also
+ *                                  holds the padding rows up to n_pad = n rounded up to a multiple of 256). The image is
+ *                                  n_pad * *image_bytes_per_row bytes and nothing may be written past that: copy every
+ *                                  GPU's part into every other GPU's image, then scema_tc_shard_commit. Any other value (2: two slices, 3: raw copies,
  *                                  0: SCEMA_PAIRS_DMMA, -1: SCEMA_PAIRS_EXACT): nothing was built, take the ordinary
  *                                  scema_compare (every GPU gets the same value).
  *        scema_tc_shard_commit  derives the second operand flavour; rows_ready_event (a cudaEvent_t as void*, may be NULL)
  *                                  is what the exact recompute of the following scema_compare(threshold, SCEMA_PAIRS_TC,
  *                                  shard, n_shards) waits for — record it behind the all-gather of the FP64 rows, which may
- *                                  then overlap the filter. scema_b200/distributed.py drives this with torch.distributed. */
+ *                                  then overlap the filter. scema_b200/distributed.py drives this with torch.distributed.
+ *      The calls must come in this order: stats, finish and commit out of turn return SCEMA_ERR_STATE, and so does commit
+ *      after a finish that chose another filter. */
 int scema_tc_shard_begin(scema_ctx *ctx, double threshold, uint64_t row0, uint64_t row1, const double **centre_dev);
 int scema_tc_shard_stats(scema_ctx *ctx, const double *centre_dev, const uint64_t **packet_dev, uint64_t *packet_words);
 int scema_tc_shard_finish(scema_ctx *ctx, const uint64_t *packets_dev, uint32_t n_shards, uint64_t pairs, int optimistic, int *choice,

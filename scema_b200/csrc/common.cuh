@@ -129,10 +129,10 @@ struct scema_ctx {
     double tc_thr = 0.0, tc_T0 = 0.0, tc_cguard = 0.0;
     bool tc_valid = false;
     bool tc_compact = false;             // hi-only operand copies (sharded prepare)
+    uint32_t shard_phase = 0;            // sharded prepare: 0 none, 1 begun, 2 statistics taken, 3 own image built (commit next)
     uint64_t shard_r0 = 0, shard_r1 = 0; // own rows of a sharded prepare
     uint64_t *h_plan = nullptr;          // pinned: survivor-density sample of a sharded prepare (read back asynchronously)
     bool plan_pending = false;
-    uint32_t plan_shards = 1;
     uint64_t plan_pairs = 0;
     bool ids_lazy = false, hist_ids_lazy = false;  // the IDs are 0 .. n-1 and the vector has not been filled (a million-entry
                                                    // refill per call is a millisecond of host time on the per-timestep path)

@@ -930,7 +930,7 @@ __global__ void __launch_bounds__(128) k_tc_prep_proj(const double *__restrict__
 // ---- survivor-density estimate ---------------------------------------------------------------------
 // PLAN_SAMPLE pseudo-random pairs, one warp each, in FP64: would the pair survive the one-slice filter, the two-slice
 // filter — each with centred and with raw operand copies — the FP64 DMMA filter and (proj != 0) the projected filter?
-// plan[0..5] receive the six counts; the host turns them into survivor estimates and picks the variant BEFORE the first launch (tc_choose),
+// plan[0..5] receive the six counts, plan[6] one per launch; the host turns them into survivor estimates and picks the variant BEFORE the first launch (tc_choose),
 // instead of finding out by overflowing the queue.
 // Criterion (DESIGN.md "K2-TC"): acc >= 0  <=>  d^2 <= c (|a'|^2 + |b'|^2) + T0 (1 + 4c) + 2 e0 / s^2, a' = a - m.
 constexpr uint32_t PLAN_SAMPLE = 8192;
@@ -948,6 +948,7 @@ __global__ void __launch_bounds__(256) k_tc_plan_sample(const double *__restrict
     const uint32_t t = blockIdx.x * 8 + (threadIdx.x >> 5);
     const int lane = threadIdx.x & 31;
     if (t >= PLAN_SAMPLE) return;
+    if (t == 0 && lane == 0) atomicAdd(misc + PLAN_WORD + 6, 1ull);   // plan[6]: samples taken (a sharded prepare sums the shards')
     // pairs among the n rows starting at r0
     const uint64_t i = r0 + plan_mix(0x5ce3a0000ull + 2 * t) % n, j = r0 + plan_mix(0x5ce3a0001ull + 2 * t) % n;
     if (i == j) return;
@@ -1290,6 +1291,7 @@ int tc_prepare_begin(scema_ctx *ctx, double thr, uint32_t slices)
     const uint64_t n_pad = (n + tc::COLT - 1) / tc::COLT * tc::COLT;
     ctx->tc_valid = false;
     ctx->tc_compact = false;  // [hi | lo] blocks unless a sharded prepare (tc_shard_*) asks for the hi-only layout
+    ctx->shard_phase = 0;     // any prepare ends a sharded one in progress
     ctx->tc_band = false;  // row order unless tc_prepare sorts by norm afterwards
     ctx->tc_proj = false;  // 64-column copies unless tc_prepare chooses the projection
     const uint32_t nc = tc_chunks(K);
@@ -1617,7 +1619,10 @@ __global__ void __launch_bounds__(256) k_tc_derive_b(const uint4 *__restrict__ H
 int tc_shard_begin(scema_ctx *ctx, double thr, uint64_t r0, uint64_t r1, const double **centre_dev)
 {
     if (!ctx->have_spline) return fail(ctx, SCEMA_ERR_STATE, "Spline is not up to date.");
-    if (!tc_supported(ctx) || r0 > r1 || r1 > ctx->n || (r0 % 128) != 0) return fail(ctx, SCEMA_ERR_INVALID, "tc_shard_begin: bad row range or row width");
+    // a share is whole 128-row blocks of the image, the last one ending at n; an empty share (the ranks past the end of
+    // a split into equal shares) may sit at any row: it builds nothing and takes no sample
+    const bool aligned = r0 == r1 || (r0 % 128 == 0 && (r1 % 128 == 0 || r1 == ctx->n));
+    if (!tc_supported(ctx) || r0 > r1 || r1 > ctx->n || !aligned) return fail(ctx, SCEMA_ERR_INVALID, "tc_shard_begin: bad row range or row width");
     int rc = tc_prepare_begin(ctx, thr, 1);
     if (rc) return rc;
     ctx->tc_band_wanted = false;
@@ -1626,13 +1631,14 @@ int tc_shard_begin(scema_ctx *ctx, double thr, uint64_t r0, uint64_t r1, const d
     ctx->shard_r1 = r1;
     rc = tc_centre_rows(ctx, r0, r1);
     if (rc) return rc;
+    ctx->shard_phase = 1;
     if (centre_dev) *centre_dev = ctx->d_tc_centre.as<double>();
     return SCEMA_OK;
 }
 
 int tc_shard_stats(scema_ctx *ctx, const double *centre_dev, const unsigned long long **packet_dev, uint64_t *packet_words)
 {
-    if (!ctx->tc_compact) return fail(ctx, SCEMA_ERR_STATE, "tc_shard_stats: no sharded prepare in progress");
+    if (ctx->shard_phase != 1) return fail(ctx, SCEMA_ERR_STATE, "tc_shard_stats: call scema_tc_shard_begin first");
     if (centre_dev && centre_dev != ctx->d_tc_centre.as<double>())
         SCEMA_CUDA(ctx, cudaMemcpyAsync(ctx->d_tc_centre.p, centre_dev, (size_t)ctx->K * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
     const uint64_t r0 = ctx->shard_r0, r1 = ctx->shard_r1;
@@ -1646,6 +1652,7 @@ int tc_shard_stats(scema_ctx *ctx, const double *centre_dev, const unsigned long
         ctx->launches++;
         SCEMA_CUDA(ctx, cudaGetLastError());
     }
+    ctx->shard_phase = 2;
     if (packet_dev) *packet_dev = ctx->d_tc_misc.as<unsigned long long>();
     if (packet_words) *packet_words = tc::MISC_WORDS;
     return SCEMA_OK;
@@ -1657,14 +1664,14 @@ int tc_shard_stats(scema_ctx *ctx, const double *centre_dev, const unsigned long
 int tc_shard_finish(scema_ctx *ctx, const unsigned long long *packets_dev, uint32_t G, uint64_t pairs, int optimistic, int *choice,
                     const void **image_dev, uint64_t *image_bytes_per_row)
 {
-    if (!ctx->tc_compact || !packets_dev || G == 0 || !choice) return fail(ctx, SCEMA_ERR_STATE, "tc_shard_finish: no sharded prepare in progress");
+    if (ctx->shard_phase != 2) return fail(ctx, SCEMA_ERR_STATE, "tc_shard_finish: call scema_tc_shard_stats first");
+    if (!packets_dev || G == 0 || !choice) return fail(ctx, SCEMA_ERR_INVALID, "tc_shard_finish: null pointer or no shards");
     unsigned long long *misc = ctx->d_tc_misc.as<unsigned long long>();
     if (!ctx->h_plan) SCEMA_CUDA(ctx, cudaMallocHost(&ctx->h_plan, 8 * sizeof(uint64_t)));
     tc::k_tc_reduce_packets<<<(tc::MISC_WORDS + 255) / 256, 256, 0, ctx->stream>>>(packets_dev, G, misc);
     ctx->launches++;
     SCEMA_CUDA(ctx, cudaMemcpyAsync(ctx->h_plan, misc + tc::PLAN_WORD, 8 * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
     ctx->plan_pending = true;
-    ctx->plan_shards = G;
     ctx->plan_pairs = pairs;
     uint64_t est = 0;
     if (!optimistic) {
@@ -1674,14 +1681,16 @@ int tc_shard_finish(scema_ctx *ctx, const unsigned long long *packets_dev, uint3
     } else {
         *choice = 1;
     }
-    if (*choice != 1) { ctx->tc_compact = false; return SCEMA_OK; }
+    if (*choice != 1) { ctx->tc_compact = false; ctx->shard_phase = 0; return SCEMA_OK; }
     ctx->tc_slices = 1;
     ctx->tc_cguard = 0.001953125;
     ctx->cand_cap = std::max<uint64_t>(ctx->cand_cap, std::max<uint64_t>(std::max<uint64_t>(1ull << 20, 32 * ctx->n), est + est / 4));
     int rc = tc_fix_scale(ctx, 0);
     const uint64_t n_pad = (ctx->n + tc::COLT - 1) / tc::COLT * tc::COLT;
-    if (!rc) rc = tc_prep_rows(ctx, ctx->shard_r0, ctx->shard_r1 == ctx->n ? n_pad : ctx->shard_r1);
+    // the share that ends at n also writes the padding rows up to n_pad; an empty share writes nothing
+    if (!rc && ctx->shard_r1 > ctx->shard_r0) rc = tc_prep_rows(ctx, ctx->shard_r0, ctx->shard_r1 == ctx->n ? n_pad : ctx->shard_r1);
     if (rc) return rc;
+    ctx->shard_phase = 3;
     if (image_dev) *image_dev = ctx->d_tc_a.p;
     if (image_bytes_per_row) *image_bytes_per_row = (uint64_t)tc_chunks(ctx->K) * 128;
     return SCEMA_OK;
@@ -1696,10 +1705,12 @@ int tc_shard_check(scema_ctx *ctx, int *choice, uint64_t *est_survivors)
     uint64_t counts[6];
     for (int i = 0; i < 6; i++) ctx->tc_plan_counts[i] = counts[i] = i < 5 ? ctx->h_plan[i] : 0;
     ctx->plan_pending = false;
+    // h_plan[6]: shares that took a sample (an empty or one-row share takes none and must not dilute the estimate)
+    const uint64_t sampled = std::max<uint64_t>(ctx->h_plan[6], 1);
     int ch = 1, centred = 1;
     uint64_t est = 0;
-    tc_choose(ctx->plan_pairs, ctx->K, counts, (uint64_t)tc::PLAN_SAMPLE * ctx->plan_shards, (uint64_t)ctx->mem_budget, true, false, &ch,
-              &centred, &est);
+    tc_choose(ctx->plan_pairs, ctx->K, counts, (uint64_t)tc::PLAN_SAMPLE * sampled, (uint64_t)ctx->mem_budget, true, false, &ch, &centred,
+              &est);
     *choice = (ch == 1 && centred) ? 1 : (ch == 1 ? 3 : ch);   // 3: one slice but raw copies -> ordinary path
     if (est_survivors) *est_survivors = est;
     return SCEMA_OK;
@@ -1707,7 +1718,8 @@ int tc_shard_check(scema_ctx *ctx, int *choice, uint64_t *est_survivors)
 
 int tc_shard_commit(scema_ctx *ctx, void *rows_ready_event)
 {
-    if (!ctx->tc_compact) return fail(ctx, SCEMA_ERR_STATE, "tc_shard_commit: no sharded prepare in progress");
+    if (ctx->shard_phase != 3) return fail(ctx, SCEMA_ERR_STATE, "tc_shard_commit: no image of a sharded prepare to commit");
+    ctx->shard_phase = 0;
     const uint64_t n_pad = (ctx->n + tc::COLT - 1) / tc::COLT * tc::COLT;
     const uint32_t nc = tc_chunks(ctx->K);
     const uint64_t chunks16 = n_pad * nc * 8;

@@ -35,11 +35,46 @@ def shard_bounds(n, world):
 
 def aligned_shard_bounds(n, world, align=2048):
     """Equal shares of a multiple of `align` rows (the last ranks take what is left): rank r owns
-    [r * per, min(n, (r + 1) * per)). Equal, aligned shares make every exchange of the sharded path an in-place
-    all-gather (row blocks, fp16 operand images). -> (per, list of (begin, end))."""
+    [r * per, min(n, (r + 1) * per)); ranks past the end get the empty share (n, n). Equal, aligned shares make every
+    exchange of the sharded path one all-gather of equal slots (row blocks, fp16 operand images: image_exchange).
+    -> (per, list of (begin, end))."""
     per = (n + world - 1) // world
     per = (per + align - 1) // align * align
     return per, [(min(n, r * per), min(n, (r + 1) * per)) for r in range(world)]
+
+
+def image_exchange(n, world):
+    """Shares and image rows of the overlapped tcgen05 path (scema_tc_shard_*, include/scema_hist.h). Rank r owns the
+    rows bounds[r] of aligned_shard_bounds and builds the image rows own[r]: its share, and for the share that ends at n
+    also the padding rows up to n_pad (n rounded up to 256); an empty share builds nothing. The all-gather moves `per`
+    rows per rank (rank r's slot starts at row r * per). The library's image holds n_pad rows only, so when world * per
+    exceeds n_pad (staged) the gather goes through a staging buffer. -> (per, bounds, n_pad, own, staged)"""
+    per, bounds = aligned_shard_bounds(n, world)
+    n_pad = (n + 255) // 256 * 256
+    own = [(b, n_pad if e == n else e) if e > b else (b, b) for b, e in bounds]
+    return per, bounds, n_pad, own, world * per > n_pad
+
+
+def gather_images(img, n, world, rank, bpr, group=None, stage=None):
+    """All-gather of the ranks' fp16 operand images into img (a byte tensor of exactly the n_pad * bpr bytes that
+    scema_tc_shard_finish promises). In place when the equal slots fill the image exactly; otherwise every rank puts
+    its rows into its slot of `stage` (world * per * bpr bytes, allocated when None or of another size), the slots are
+    gathered there and the first n_pad rows copied into the image. -> the staging buffer (None when in place)."""
+    per, _, n_pad, own, staged = image_exchange(n, world)
+    if img.numel() != n_pad * bpr:
+        raise ValueError(f"gather_images: image of {img.numel()} bytes, expected {n_pad} rows of {bpr}")
+    slot = per * bpr
+    if not staged:
+        dist.all_gather_into_tensor(img, img[rank * slot:(rank + 1) * slot], group=group)
+        return None
+    if stage is None or stage.numel() != world * slot:
+        stage = torch.empty(world * slot, dtype=torch.uint8, device=img.device)
+    b, e = own[rank]
+    mine = stage[rank * slot:(rank + 1) * slot]
+    mine[:(e - b) * bpr].copy_(img[b * bpr:e * bpr])
+    dist.all_gather_into_tensor(stage, mine, group=group)
+    img.copy_(stage[:n_pad * bpr])
+    return stage
 
 
 def gather_rows(local_rows, n, world, group=None, bounds=None):
@@ -109,6 +144,7 @@ class ShardedCluster:
         self._side_stream = None
         self._main = None
         self._packets = None
+        self._stage = None
         self._views = {}
         self._peers = None
         self._flag = None
@@ -152,7 +188,7 @@ class ShardedCluster:
         exact recompute waits for the FP64 rows. Falls back to the plain sequence when the survivor sample prefers
         another filter. -> (local_edge_count, counts, offsets, full_rows tensor)."""
         hc, G = self.hc, self.world
-        per, bounds = aligned_shard_bounds(n, G)
+        per, bounds, n_pad, _, _ = image_exchange(n, G)
         b, e = bounds[self.rank]
         if self._main is None:
             self._main = self.stream()
@@ -204,8 +240,8 @@ class ShardedCluster:
             optimistic = self._last_choice == 1
             choice, img_ptr, bpr = hc.tc_shard_finish(self._packets.data_ptr(), G, n * (n - 1) // 2 // G, optimistic)
             if choice == 1:
-                img = self._view(img_ptr, (G * per * bpr,), "|u1")
-                dist.all_gather_into_tensor(img, img[self.rank * per * bpr:(self.rank + 1) * per * bpr], group=self.group)
+                img = self._view(img_ptr, (n_pad * bpr,), "|u1")
+                self._stage = gather_images(img, n, G, self.rank, bpr, self.group, self._stage)
                 hc.tc_shard_commit(rows_ready.cuda_event)
                 self.path = "overlapped"
             else:
