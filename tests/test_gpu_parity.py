@@ -282,12 +282,15 @@ def test_compare_stream_concatenates_to_compare(hc, vname, variant):
         tot = hc.compare_stream(THR, lambda a, b, d: chunks.append((a, b, d)), variant, panels_per_chunk=ppc)
         got = tuple(np.concatenate([c[k] for c in chunks]) for k in range(3))
         assert tot == ne and edges_equal(got, want), ppc
+        if variant == PAIRS_TC:   # config-4-shaped rows: the streamed compare runs the projected filter
+            assert hc.tc_last_plan()["projected_chosen"] and hc.counters()["tc_slices"] == 1, ppc
         if ppc == 1:
             assert len(chunks) >= 4
             assert all(chunks[i][0].max() < chunks[i + 1][0].min() for i in range(len(chunks) - 1))
     parts = []
     for shard in range(3):
         hc.compare_stream(THR, lambda a, b, d: parts.append((a, b, d)), variant, shard=shard, n_shards=3, panels_per_chunk=2)
+        assert variant != PAIRS_TC or hc.tc_last_plan()["projected_chosen"], shard
     a = np.concatenate([c[0] for c in parts]); b = np.concatenate([c[1] for c in parts]); d = np.concatenate([c[2] for c in parts])
     o = np.lexsort((b, a))
     assert edges_equal((a[o], b[o], d[o]), want)
@@ -327,6 +330,8 @@ def test_sharded_compare_union(hc, oracle):
                 hc.set_spline(rows)
                 hc.compare(THR, variant, shard=r, n_shards=world)
                 parts.append(hc.get_edges())
+                if variant == PAIRS_TC:   # every shard takes the projected filter on these rows
+                    assert hc.tc_last_plan()["projected_chosen"] and hc.counters()["tc_slices"] == 1, (world, r)
             a = np.concatenate([p[0] for p in parts])
             b = np.concatenate([p[1] for p in parts])
             d = np.concatenate([p[2] for p in parts])

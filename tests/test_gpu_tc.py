@@ -324,18 +324,21 @@ def test_tc_threshold_change_rebuilds_operands(hc, oracle):
 
 def test_tc_single_cta_kernel_and_pinned_slices_match(tmp_path):
     """SCEMA_TC_CG=1 selects the single-CTA kernel (128 x 256 tile per SM; the default is cta_group::2, an SM pair per
-    256 x 256 tile), SCEMA_TC_SLICES pins the number of fp16 slices; every combination emits the exact kernel's edge list."""
+    256 x 256 tile), SCEMA_TC_SLICES pins the number of fp16 slices (3: the projected 16-column filter); every
+    combination emits the exact kernel's edge list."""
     code = (
         "import numpy as np, scema_b200\n"
         "from scema_b200 import synth, PAIRS_TC, PAIRS_EXACT\n"
         "rows = synth.rows(31, 7000, 16, 10, 5e-3, synth.default_pert(1e-6, 10))\n"
         "hc = scema_b200.HistCluster(0); hc.set_spline(rows)\n"
-        "n1 = hc.compare(1e-6, PAIRS_TC); e1 = hc.get_edges(); assert hc.counters()['tc_slices'] == int(__import__('os').environ['SCEMA_TC_SLICES'])\n"
+        "pin = int(__import__('os').environ['SCEMA_TC_SLICES'])\n"
+        "n1 = hc.compare(1e-6, PAIRS_TC); e1 = hc.get_edges(); assert hc.counters()['tc_slices'] == (1 if pin == 3 else pin)\n"
+        "assert hc.tc_last_plan()['projected_chosen'] == (pin == 3)\n"
         "n2 = hc.compare(1e-6, PAIRS_EXACT); e2 = hc.get_edges()\n"
         "assert n1 == n2 and n1 > 7000\n"
         "assert all(np.array_equal(x.view(np.uint64) if x.dtype == np.float64 else x, y.view(np.uint64) if y.dtype == np.float64 else y) for x, y in zip(e1, e2))\n"
         "print('ok', n1)\n")
-    for cg, sl in (("1", "1"), ("1", "2"), ("2", "1"), ("2", "2")):
+    for cg, sl in (("1", "1"), ("1", "2"), ("1", "3"), ("2", "1"), ("2", "2"), ("2", "3")):
         env = dict(os.environ, SCEMA_TC_CG=cg, SCEMA_TC_SLICES=sl, PYTHONPATH=ROOT)
         r = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=300)
         assert r.returncode == 0 and r.stdout.startswith("ok"), (cg, sl, r.stdout, r.stderr)
