@@ -172,6 +172,46 @@ int scema_knn(scema_ctx *ctx, uint32_t k, int variant, uint32_t *index_host, dou
  * (0 for rounds not run). Either pointer may be NULL. */
 int scema_knn_last_stats(scema_ctx *ctx, uint64_t counts[8], double radii[8]);
 
+/* ---- cross queries: a second set of m histories (the queries) against the current spline matrix (the retained
+ *      histories), the question compare_histories_with_all_ranks (strain2spline.h:590-598) asks on every ring step after
+ *      the first. rows = the queries [m][k_cols], already resampled (row layout p*6+c, as scema_get_spline), in host
+ *      memory, or on the device with rows_on_device (borrowed for the duration of the call only; for raw histories,
+ *      resample them on a second context and pass scema_spline_info's device pointer). Index i is the batch index of a
+ *      retained history (also after scema_select_rows and on the store path), index j the position in the query array. A
+ *      query is never "itself": a query equal to a retained row is listed at distance 0. (a - b)^2 and (b - a)^2 round
+ *      identically, so every diff has the bits of compare_L2_norm(row i, query j). Every variant gives the identical
+ *      result. SCEMA_ERR_INVALID: k_cols != the matrix's k, a bad variant, k outside [1, 32], m > 0 with rows == NULL,
+ *      n + m >= 2^32; SCEMA_ERR_STATE without a spline matrix. m = 0 or n = 0 give an empty result. Both calls run on a
+ *      private context: the last compare of this context (edges, degrees, timings, counters, audit, operand caches) and
+ *      scema_knn_last_stats are left exactly as they were, also when the call fails. Memory: the scratch copy [Q; R] of
+ *      (m + n) rows, plus the edges of its first ceil(m / 2048) row panels.
+ *
+ * scema_query_compare: every pair (query j, history i) with compare_L2_norm(i, j) < threshold (thresholds <= 0 or NaN:
+ * none), sorted by (j, i). *n_edges = their number. scema_query_get_edges copies the first cap of them to host arrays (any
+ * pointer may be NULL). They stay readable until the next scema_query_compare on this context, which replaces them (a
+ * failed one leaves none: SCEMA_ERR_STATE); scema_compare, scema_knn, scema_query_knn and new spline matrices do not touch
+ * them. */
+int scema_query_compare(scema_ctx *ctx, const double *rows, int rows_on_device, uint64_t m, uint32_t k_cols, double threshold,
+                        int variant, uint64_t *n_edges);
+int scema_query_get_edges(scema_ctx *ctx, uint32_t *query_index, uint32_t *row_index, double *diff, uint64_t cap);
+/* scema_query_knn: the k nearest retained histories of every query: slots [j*k, j*k + k) of both host arrays (either may
+ * be NULL), ordered by (diff, ids[i], i) as scema_knn; NaN partners skipped, +inf listed, empty slots {UINT32_MAX, +inf}.
+ * The rounds of scema_knn with the queries as the rows: a radius from the open queries sampled against a seeded subset
+ * of the matrix, a compare of [open queries; matrix] that closes every query with k partners below it, and the exact
+ * top-k kernel for what is left (all queries with SCEMA_PAIRS_EXACT, or when open queries * n <= 2^28). */
+int scema_query_knn(scema_ctx *ctx, const double *rows, int rows_on_device, uint64_t m, uint32_t k_cols, uint32_t k, int variant,
+                    uint32_t *index_host, double *diff_host);
+/* The last scema_query_*: counts = {filter rounds run, queries finished in round 1, queries finished in later rounds,
+ * queries finished by the exact kernel, pairs the exact kernel evaluated, filter survivors, edges of the [Q; R] prefix
+ * compares (all of them: also query x query and the retained rows that share the last query panel), filter variant of
+ * the last round (SCEMA_PAIRS_EXACT when none ran), pairs of the row panels the filter was launched on (at most
+ * m n + m (m - 1) / 2 + 2048 n per round), cross edges (scema_query_compare), passes of the compares (more than one
+ * per round: a queue or edge buffer overflowed and the compare grew it or re-decided its filter)}; radii = the threshold /
+ * the radius of each round; ms = CUDA-event milliseconds of {scratch copy [Q; R] (with the upload of host queries),
+ * operand prep, filter, exact recompute, sort, compaction / selection of the cross entries, exact top-k kernel, 0}. Any
+ * pointer may be NULL. */
+int scema_query_last_stats(scema_ctx *ctx, uint64_t counts[11], double radii[8], float ms[8]);
+
 /* One call for a host caller: set_histories + resample + compare. With SCEMA_PAIRS_TC, 6 * spline_points <= 60
  * and a large batch (>= 65536 histories; SCEMA_PIPELINE=0 disables, SCEMA_PIPELINE_MIN_N moves the limit) the three
  * steps are pipelined range by range behind the host->device copy of the raw steps: range c is resampled and compared

@@ -59,6 +59,10 @@ def lib():
         "scema_nearest": (i32, [vp, vp, vp]),
         "scema_knn": (i32, [vp, u32, i32, vp, vp]),
         "scema_knn_last_stats": (i32, [vp, vp, vp]),
+        "scema_query_compare": (i32, [vp, vp, i32, u64, u32, dbl, i32, P(u64)]),
+        "scema_query_get_edges": (i32, [vp, vp, vp, vp, u64]),
+        "scema_query_knn": (i32, [vp, vp, i32, u64, u32, u32, i32, vp, vp]),
+        "scema_query_last_stats": (i32, [vp, vp, vp, vp]),
         "scema_write_similar_hist": (i32, [vp, C.c_char_p]),
         "scema_reduce_edges": (i32, [vp, u32, vp, P(u64), P(u64)]),
         "scema_reduce_calls": (i32, [vp, vp, u64, u32, vp, P(u64), P(u64)]),
@@ -123,7 +127,8 @@ EXPORTED = (
     "scema_create scema_destroy scema_last_error scema_version scema_stream scema_set_histories scema_resample "
     "scema_store_reset scema_store_append scema_store_info scema_store_resample scema_select_rows "
     "scema_set_spline scema_get_spline scema_spline_info scema_compare scema_compare_stream scema_get_edges scema_edges_device "
-    "scema_get_degrees scema_cluster scema_nearest scema_knn scema_knn_last_stats scema_write_similar_hist scema_reduce_edges scema_reduce_calls scema_reduce_dir "
+    "scema_get_degrees scema_cluster scema_nearest scema_knn scema_knn_last_stats "
+    "scema_query_compare scema_query_get_edges scema_query_knn scema_query_last_stats scema_write_similar_hist scema_reduce_edges scema_reduce_calls scema_reduce_dir "
     "scema_last_timings scema_last_counters scema_kernel_launches scema_last_audit scema_fp64_peak scema_k1_tune scema_tc_debug scema_tc_plan scema_tc_shard_begin scema_tc_shard_stats scema_tc_shard_finish scema_tc_shard_check scema_tc_shard_commit scema_tc_centre scema_tc_last_plan scema_tc_choose scema_tc_choose_projected scema_tc_basis scema_tc_last_projection scema_pipeline_plan scema_synth_offsets "
     "scema_multi_create scema_multi_destroy scema_multi_last_error scema_multi_devices scema_multi_context scema_multi_cluster "
     "scema_multi_compare_rows scema_multi_shard_edges scema_multi_last_ms "
@@ -440,6 +445,62 @@ class HistCluster:
         return {"rounds": int(c[0]), "rows_round1": int(c[1]), "rows_later_rounds": int(c[2]), "rows_exact": int(c[3]),
                 "exact_pairs": int(c[4]), "survivors": int(c[5]), "edges": int(c[6]), "variant": int(c[7]),
                 "radii": [float(x) for x in r][:int(c[0])]}
+
+    def _query_rows(self, rows, device_ptr, m, k_cols):
+        """-> (pointer, on_device, m, k_cols, keep-alive) of the query rows: a host array [m, k_cols], or device_ptr with m
+        and k_cols (k_cols defaults to the matrix's)."""
+        if device_ptr is not None:
+            if m is None:
+                raise ValueError("query rows on the device: pass their number as m")
+            if k_cols is None:
+                k_cols = self.spline_info()[1]
+            return int(device_ptr), 1, int(m), int(k_cols), None
+        rows = np.ascontiguousarray(rows, dtype=np.float64)
+        if rows.ndim != 2:
+            raise ValueError("query rows: a 2-d array [m, k]")
+        return _ptr(rows) if rows.size else None, 0, rows.shape[0], rows.shape[1], rows
+
+    def query_compare(self, rows, threshold, variant=PAIRS_TC, device_ptr=None, m=None, k_cols=None):
+        """Every (query j, history i) with compare_L2_norm < threshold, sorted by (j, i): (query_index, row_index, diff).
+        rows: host array [m, k]; or device_ptr=int with m (and k_cols) for device-resident rows."""
+        p, dev, m, k_cols, keep = self._query_rows(rows, device_ptr, m, k_cols)
+        ne = C.c_uint64(0)
+        self._ck(self._L.scema_query_compare(self._h, p, dev, m, k_cols, float(threshold), int(variant), C.byref(ne)))
+        del keep
+        return self.query_edges(int(ne.value))
+
+    def query_edges(self, count):
+        """The first `count` cross edges of the last query_compare."""
+        j = np.empty(count, dtype=np.uint32)
+        i = np.empty(count, dtype=np.uint32)
+        d = np.empty(count, dtype=np.float64)
+        self._ck(self._L.scema_query_get_edges(self._h, _ptr(j), _ptr(i), _ptr(d), count))
+        return j, i, d
+
+    def query_knn(self, rows, k, variant=PAIRS_TC, device_ptr=None, m=None, k_cols=None):
+        """The k nearest histories of every query row: (index [m, k] uint32, diff [m, k] float64), slots in order of
+        (diff, ID, index); empty slots are (0xffffffff, inf)."""
+        p, dev, m, k_cols, keep = self._query_rows(rows, device_ptr, m, k_cols)
+        kk = max(int(k), 0)
+        index = np.empty((m, kk), dtype=np.uint32)
+        diff = np.empty((m, kk), dtype=np.float64)
+        self._ck(self._L.scema_query_knn(self._h, p, dev, m, k_cols, int(k) & 0xffffffff, int(variant), _ptr(index), _ptr(diff)))
+        del keep
+        return index, diff
+
+    def query_last_stats(self):
+        """What the last query_compare / query_knn did: rounds, queries finished per stage, exact pairs, survivors, edges of
+        the prefix compares, last filter variant, filter pairs, cross edges, compare passes, the radius of every round and the phase
+        times (ms)."""
+        c = (C.c_uint64 * 11)()
+        r = (C.c_double * 8)()
+        t = (C.c_float * 8)()
+        self._ck(self._L.scema_query_last_stats(self._h, c, r, t))
+        names = ("copy", "prep", "filter", "exact", "sort", "select", "topk")
+        return {"rounds": int(c[0]), "rows_round1": int(c[1]), "rows_later_rounds": int(c[2]), "rows_exact": int(c[3]),
+                "exact_pairs": int(c[4]), "survivors": int(c[5]), "edges": int(c[6]), "variant": int(c[7]),
+                "filter_pairs": int(c[8]), "cross_edges": int(c[9]), "passes": int(c[10]), "radii": [float(x) for x in r][:max(int(c[0]), 1)],
+                "ms": {names[w]: float(t[w]) for w in range(len(names))}}
 
     def cluster(self, steps, offsets, ids, spline_points, threshold, variant=PAIRS_TC):
         steps = np.ascontiguousarray(steps, dtype=np.float64)

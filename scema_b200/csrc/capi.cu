@@ -69,6 +69,9 @@ void scema_destroy(scema_ctx *c)
     if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
     if (c->knn_child) scema_destroy(c->knn_child);
     for (scema::DevBuf &b : c->knn_buf) b.release();
+    if (c->query_child) scema_destroy(c->query_child);
+    c->query_j.release(); c->query_i.release(); c->query_d.release();
+    for (cudaEvent_t e : c->query_ev) if (e) cudaEventDestroy(e);
     if (c->own_stream) cudaStreamDestroy(c->stream);
     delete c;
 }
@@ -351,6 +354,48 @@ int scema_knn_last_stats(scema_ctx *c, uint64_t counts[8], double radii[8])
     for (int i = 0; i < 8; i++) {
         if (counts) counts[i] = c->knn_counts[i];
         if (radii) radii[i] = c->knn_radii[i];
+    }
+    return SCEMA_OK;
+}
+
+int scema_query_compare(scema_ctx *c, const double *rows, int rows_on_device, uint64_t m, uint32_t k_cols, double threshold, int variant,
+                        uint64_t *n_edges)
+{
+    int rc = enter(c);
+    if (rc) return rc;
+    return query_compare_run(c, rows, rows_on_device, m, k_cols, threshold, variant, n_edges);
+}
+
+int scema_query_get_edges(scema_ctx *c, uint32_t *query_index, uint32_t *row_index, double *diff, uint64_t cap)
+{
+    int rc = enter(c);
+    if (rc) return rc;
+    if (!c->have_query) return fail(c, SCEMA_ERR_STATE, "query_get_edges: no scema_query_compare result");
+    const uint64_t m = std::min<uint64_t>(cap, c->query_n);
+    if (m == 0) return SCEMA_OK;
+    if (query_index) SCEMA_CUDA(c, cudaMemcpyAsync(query_index, c->query_j.p, m * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+    if (row_index) SCEMA_CUDA(c, cudaMemcpyAsync(row_index, c->query_i.p, m * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+    if (diff) SCEMA_CUDA(c, cudaMemcpyAsync(diff, c->query_d.p, m * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    SCEMA_CUDA(c, cudaStreamSynchronize(c->stream));
+    return SCEMA_OK;
+}
+
+int scema_query_knn(scema_ctx *c, const double *rows, int rows_on_device, uint64_t m, uint32_t k_cols, uint32_t k, int variant,
+                    uint32_t *index_host, double *diff_host)
+{
+    int rc = enter(c);
+    if (rc) return rc;
+    return query_knn_run(c, rows, rows_on_device, m, k_cols, k, variant, index_host, diff_host);
+}
+
+int scema_query_last_stats(scema_ctx *c, uint64_t counts[11], double radii[8], float ms[8])
+{
+    if (!c) return SCEMA_ERR_INVALID;
+    for (int i = 0; i < 11; i++)
+        if (counts) counts[i] = c->query_counts[i];
+    for (int i = 0; i < 8; i++) {
+        if (radii) radii[i] = c->query_radii[i];
+        if (ms) ms[i] = c->query_ms[i];
     }
     return SCEMA_OK;
 }

@@ -169,9 +169,20 @@ struct scema_ctx {
     // ---- scema_knn (knn.cu): the filter rounds run on a private child context (on the same device and stream) so that
     //      this context's compare results stay as they are; scratch buffers and the stats of the last call
     scema_ctx *knn_child = nullptr;
-    scema::DevBuf knn_buf[16];
+    scema::DevBuf knn_buf[16];  // scratch of scema_knn and the scema_query_* calls (nothing in it outlives a call)
     uint64_t knn_counts[8] = {};
     double knn_radii[8] = {};
+
+    // ---- scema_query_compare / scema_query_knn (knn.cu): their own child context, so that a query leaves the state of
+    //      scema_knn's child (queue sizes, filter decisions) as it was; the cross edges of the last scema_query_compare
+    scema_ctx *query_child = nullptr;
+    scema::DevBuf query_j, query_i, query_d;
+    uint64_t query_n = 0;
+    bool have_query = false;
+    uint64_t query_counts[11] = {};
+    double query_radii[8] = {};
+    float query_ms[8] = {};
+    cudaEvent_t query_ev[2] = {nullptr, nullptr};
 };
 
 namespace scema {
@@ -233,7 +244,7 @@ int compare_stream_run(scema_ctx *ctx, double thr, int variant, uint32_t shard, 
                        scema_edge_sink sink, void *user, uint64_t *n_total);
 int fp64_peak_run(scema_ctx *ctx, double out[2]);
 int nearest_run(scema_ctx *ctx, uint32_t *nearest_id_host, double *nearest_diff_host);
-int compare_prefix_run(scema_ctx *ctx, double thr, int *variant, uint32_t p1);
+int compare_prefix_run(scema_ctx *ctx, double thr, int *variant, uint32_t p1, bool plan_prefix);
 int edges_adopt(scema_ctx *ctx, const uint64_t *d_keys, const double *d_vals, uint64_t total);
 bool pipeline_wanted(uint64_t n);
 void pipeline_bounds(uint64_t n, std::vector<uint64_t> &bounds);
@@ -270,6 +281,10 @@ int tc_debug_run(scema_ctx *ctx, double thr, uint32_t slices, float *acc_host, u
                  unsigned char *hb_host);
 // knn.cu
 int knn_run(scema_ctx *ctx, uint32_t k, int variant, uint32_t *index_host, double *diff_host);
+int query_compare_run(scema_ctx *ctx, const double *rows, int rows_on_device, uint64_t m, uint32_t k_cols, double thr, int variant,
+                      uint64_t *n_edges);
+int query_knn_run(scema_ctx *ctx, const double *rows, int rows_on_device, uint64_t m, uint32_t k_cols, uint32_t k, int variant,
+                  uint32_t *index_host, double *diff_host);
 // host_io.cc
 int write_similar_hist(scema_ctx *ctx, const char *pattern);
 int reduce_graph_calls(const uint32_t *eu, const uint32_t *ev, uint64_t n_calls, uint32_t num_gps,

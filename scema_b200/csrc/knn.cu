@@ -10,6 +10,12 @@
 // evaluates the open rows against all n rows. The rounds run on a private child context so that the caller's compare
 // results, timings and operand caches stay untouched.
 //
+// scema_query_knn runs the same rounds for the rows of a second set (the queries) against the matrix: every round samples
+// the open queries against the subset, stacks [open queries; matrix] on a private child context, and compares the prefix
+// panels [0, ceil(|U| / 2048)), which hold every query x matrix pair; only those entries count. scema_query_compare is
+// one such compare at the caller's threshold, with the cross edges compacted out of the prefix's list (DESIGN.md "Cross
+// query").
+//
 // Order of the k slots: (diff, ID, index) ascending; non-negative doubles order as their bit patterns, so a slot is
 // keyed by (bits, ID, index) and every kernel below keeps the k smallest keys under that total order — the result does
 // not depend on the order in which candidates arrive.
@@ -30,6 +36,7 @@ constexpr double KNN_QUANTILE_C = 2.0;           // radius: the sampled fraction
 constexpr uint64_t KNN_QUANTILE_MIN = 16;        // ... and at least this many sampled distances lie below it
 constexpr int KNN_MAX_ROUNDS = 4;                // filter rounds at most
 constexpr double KNN_EXACT_PAIRS = 2147483648.0; // |U| * n at or below this: the open rows go to k_knn_exact
+constexpr double KNN_QUERY_EXACT_PAIRS = 268435456.0;  // scema_query_knn: open queries * n at or below this go to k_knn_exact
 constexpr double KNN_EDGE_BUDGET = 8.0;          // a round whose estimated edges exceed this * n * k (+ 2^20) is not run
 constexpr uint64_t KNN_MIN_N = 2048;             // fewer rows (one panel): k_knn_exact for all of them
 constexpr uint64_t KNN_SEED = 0x6b6e6e5eedull;   // seed of the subset
@@ -79,21 +86,23 @@ __device__ __forceinline__ void topk_offer(TopK &t, uint32_t k, bool valid, unsi
 }
 
 // ------------------------------------------------------------------------------------------------
-// k_knn_exact: the query rows q_rows[0, nq) against the columns of segment blockIdx.y, one query row per warp, tiles of
-// 64 columns (two per lane) staged through shared memory in slices of 32 of the K entries, sums in the reference's
-// order (k_exact_all's arithmetic; a - b and b - a round to the same magnitude). Writes each (query, segment)'s k best.
+// k_knn_exact: the query rows Q[q_rows[0, nq)] against the columns S[0, n) of segment blockIdx.y, one query row per warp,
+// tiles of 64 columns (two per lane) staged through shared memory in slices of 32 of the K entries, sums in the
+// reference's order (k_exact_all's arithmetic; a - b and b - a round to the same magnitude). Writes each (query,
+// segment)'s k best. self: Q == S and a query row is not its own neighbour (scema_knn); 0: a second set (scema_query_knn).
 // ------------------------------------------------------------------------------------------------
 constexpr int KQ = 8, KCOL = 64, KKC = 32;
 __global__ void __launch_bounds__(256, 4) k_knn_exact(const double *__restrict__ S, uint64_t n, uint32_t K, const uint32_t *__restrict__ ids,
-                                                   const uint32_t *__restrict__ q_rows, uint32_t nq, uint64_t seg_len, uint32_t k,
-                                                   unsigned long long *__restrict__ part_b, uint32_t *__restrict__ part_ix)
+                                                   const double *__restrict__ Q, const uint32_t *__restrict__ q_rows, uint32_t nq, int self,
+                                                   uint64_t seg_len, uint32_t k, unsigned long long *__restrict__ part_b,
+                                                   uint32_t *__restrict__ part_ix)
 {
     __shared__ double Qs[KQ][KKC];
     __shared__ double Cs[KCOL][KKC + 1];
     const int tid = threadIdx.x, w = tid >> 5, lane = tid & 31;
     const uint32_t qp = blockIdx.x * KQ + w;
     const bool have_q = qp < nq;
-    const uint32_t qrow = have_q ? q_rows[qp] : 0xffffffffu;  // n < 2^32: no column has this index
+    const uint32_t qrow = have_q && self ? q_rows[qp] : 0xffffffffu;  // n < 2^32 - 1: no column has this index
     const uint64_t c_begin = (uint64_t)blockIdx.y * seg_len, c_end = n < c_begin + seg_len ? n : c_begin + seg_len;
     TopK t;
     for (uint64_t c0 = c_begin; c0 < c_end; c0 += KCOL) {
@@ -104,7 +113,7 @@ __global__ void __launch_bounds__(256, 4) k_knn_exact(const double *__restrict__
             {
                 const int r = tid / KKC, kk = tid - r * KKC;  // KQ * KKC == 256: one entry per thread
                 const uint32_t q = blockIdx.x * KQ + r;
-                Qs[r][kk] = (q < nq && (uint32_t)kk < kn) ? S[(uint64_t)q_rows[q] * K + k0 + kk] : 0.0;
+                Qs[r][kk] = (q < nq && (uint32_t)kk < kn) ? Q[(uint64_t)q_rows[q] * K + k0 + kk] : 0.0;
             }
             for (int e = tid; e < KCOL * KKC; e += 256) {
                 const int r = e / KKC, kk = e - r * KKC;
@@ -178,18 +187,29 @@ __global__ void __launch_bounds__(256) k_knn_topk(const unsigned long long *__re
 
 // Directed entries of a round's edges (a < b, indices into the round's matrix; perm maps them to rows of the caller's
 // matrix, nullptr = identity) for the rows that are still open. PASS 0 counts per row, PASS 1 scatters (cursor = offsets).
+// cross > 0 (scema_query_knn): the round's matrix is [open queries; retained rows] with `cross` queries in front; only the
+// query -> retained entries (a < cross <= b) count, as (perm[a], b - cross).
 template <int PASS>
 __global__ void __launch_bounds__(256) k_knn_expand(const uint64_t *__restrict__ keys, const double *__restrict__ vals, uint64_t m,
-                                                    uint32_t key_shift, const uint32_t *__restrict__ perm, const uint8_t *__restrict__ open,
-                                                    unsigned long long *__restrict__ cnt_or_cursor, unsigned long long *__restrict__ eb,
-                                                    uint32_t *__restrict__ eix)
+                                                    uint32_t key_shift, const uint32_t *__restrict__ perm, uint64_t cross,
+                                                    const uint8_t *__restrict__ open, unsigned long long *__restrict__ cnt_or_cursor,
+                                                    unsigned long long *__restrict__ eb, uint32_t *__restrict__ eix)
 {
     const uint64_t e = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= m) return;
     const uint64_t key = keys[e];
     uint32_t a = (uint32_t)(key >> key_shift), b = (uint32_t)(key & ((1ull << key_shift) - 1));
-    if (perm) { a = perm[a]; b = perm[b]; }
     const unsigned long long bits = (unsigned long long)__double_as_longlong(vals[e]);
+    if (cross) {
+        if (!(a < cross && b >= cross)) return;
+        const uint32_t q = perm[a];
+        if (open[q]) {
+            const unsigned long long o = atomicAdd(cnt_or_cursor + q, 1ull);
+            if (PASS == 1) { eb[o] = bits; eix[o] = b - (uint32_t)cross; }
+        }
+        return;
+    }
+    if (perm) { a = perm[a]; b = perm[b]; }
     if (open[a]) {
         const unsigned long long o = atomicAdd(cnt_or_cursor + a, 1ull);
         if (PASS == 1) { eb[o] = bits; eix[o] = b; }
@@ -200,10 +220,12 @@ __global__ void __launch_bounds__(256) k_knn_expand(const uint64_t *__restrict__
     }
 }
 
-// Distance sample: rows A (rows_a[a * a_span / na], a < na) against rows B; tri: only b > a (A == B). Same-row pairs and
-// NaN distances are left out. Bits appended with one atomic per warp.
-__global__ void __launch_bounds__(256) k_knn_sample(const double *__restrict__ S, uint32_t K, const uint32_t *__restrict__ rows_a,
-                                                    uint32_t na, uint64_t a_span, const uint32_t *__restrict__ rows_b, uint32_t nb, int tri,
+// Distance sample: rows A (SA[rows_a[a * a_span / na]], a < na) against rows B (S[rows_b[b]]); tri: only b > a (A == B).
+// Same-row pairs (unless cross: A is another set than B) and NaN distances are left out. Bits appended with one atomic
+// per warp.
+__global__ void __launch_bounds__(256) k_knn_sample(const double *__restrict__ S, const double *__restrict__ SA, int cross, uint32_t K,
+                                                    const uint32_t *__restrict__ rows_a, uint32_t na, uint64_t a_span,
+                                                    const uint32_t *__restrict__ rows_b, uint32_t nb, int tri,
                                                     unsigned long long *__restrict__ out, unsigned long long *__restrict__ count)
 {
     const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -212,8 +234,8 @@ __global__ void __launch_bounds__(256) k_knn_sample(const double *__restrict__ S
     unsigned long long bits = 0;
     if (a < na && !(tri && b <= a)) {
         const uint32_t i = rows_a[(uint64_t)a * a_span / na], j = rows_b[b];
-        if (i != j) {
-            const double d = exact_l2(S + (uint64_t)i * K, S + (uint64_t)j * K, K);
+        if (cross || i != j) {
+            const double d = exact_l2(SA + (uint64_t)i * K, S + (uint64_t)j * K, K);
             keep = d == d;
             bits = (unsigned long long)__double_as_longlong(d);
         }
@@ -250,19 +272,90 @@ __global__ void __launch_bounds__(256) k_knn_gather(const double *__restrict__ S
 }
 
 // ------------------------------------------------------------------------------------------------
+// scema_query_compare: the cross edges of a [Q; R] prefix compare. The child's sorted edges (a, b), a < b, of the stacked
+// matrix are kept when a < m <= b (query a, retained row b - m), in order, so the list stays sorted by (j, i).
+// flag[ne] = 0 so that the exclusive sum's last entry is the number kept.
+// ------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) k_query_flag(const uint64_t *__restrict__ keys, uint64_t ne, uint32_t key_shift, uint64_t m,
+                                                    unsigned long long *__restrict__ flag)
+{
+    const uint64_t e = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e > ne) return;
+    if (e == ne) { flag[e] = 0; return; }
+    const uint64_t key = keys[e];
+    const uint64_t a = key >> key_shift, b = key & ((1ull << key_shift) - 1);
+    flag[e] = a < m && b >= m;
+}
+
+__global__ void __launch_bounds__(256) k_query_scatter(const uint64_t *__restrict__ keys, const double *__restrict__ vals, uint64_t ne,
+                                                       uint32_t key_shift, uint64_t m, const unsigned long long *__restrict__ flag,
+                                                       const unsigned long long *__restrict__ pos, uint32_t *__restrict__ out_j,
+                                                       uint32_t *__restrict__ out_i, double *__restrict__ out_d)
+{
+    const uint64_t e = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= ne || !flag[e]) return;
+    const uint64_t key = keys[e], o = pos[e];
+    out_j[o] = (uint32_t)(key >> key_shift);
+    out_i[o] = (uint32_t)((key & ((1ull << key_shift) - 1)) - m);
+    out_d[o] = vals[e];
+}
+
+// ------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------
 namespace {
 
-enum { B_IDS, B_OPEN, B_PERM, B_OUT_IX, B_OUT_D, B_SUBSET, B_SAMPLE, B_TMP, B_MISC, B_CNT, B_EB, B_EIX, B_ROWS, B_PART_B, B_PART_IX };
+enum { B_IDS, B_OPEN, B_PERM, B_OUT_IX, B_OUT_D, B_SUBSET, B_SAMPLE, B_TMP, B_MISC, B_CNT, B_EB, B_EIX, B_ROWS, B_PART_B, B_PART_IX, B_Q };
 
+// Phases of the query calls, timed with the context's query events (the compare events belong to the last compare).
+enum { QT_COPY, QT_PREP, QT_FILTER, QT_EXACT, QT_SORT, QT_SELECT, QT_TOPK };
+
+// Events around a stretch of work on the caller's stream, folded into query_ms[which] (host-synchronising); on = false
+// (scema_knn, which reports no phases) records nothing.
+struct QTimer {
+    scema_ctx *c;
+    int which;
+    bool on;
+    QTimer(scema_ctx *ctx, int w, bool on_) : c(ctx), which(w), on(on_) { if (on) cudaEventRecord(c->query_ev[0], c->stream); }
+    void stop()
+    {
+        if (!on) return;
+        cudaEventRecord(c->query_ev[1], c->stream);
+        float t = 0.f;
+        if (cudaEventSynchronize(c->query_ev[1]) == cudaSuccess && cudaEventElapsedTime(&t, c->query_ev[0], c->query_ev[1]) == cudaSuccess)
+            c->query_ms[which] += t;
+        else
+            cudaGetLastError();
+    }
+};
+
+// Seeded stratified subset: one row from each of S equal slices of [0, n).
+void make_subset(uint64_t n, std::vector<uint32_t> &out)
+{
+    const uint64_t s = std::min<uint64_t>(n, KNN_SAMPLE_ROWS);
+    out.resize(s);
+    for (uint64_t i = 0; i < s; i++) {
+        uint64_t z = KNN_SEED + 0x9e3779b97f4a7c15ull * (i + 1);
+        z = (z ^ (z >> 30)) * 0xbf58476d1ce4e5b9ull;
+        z = (z ^ (z >> 27)) * 0x94d049bb133111ebull;
+        z ^= z >> 31;
+        const uint64_t lo = i * n / s, hi = (i + 1) * n / s;
+        out[i] = (uint32_t)(lo + z % (hi - lo));
+    }
+}
+
+// The k nearest of `rows` listed rows among the n rows of the caller's matrix. scema_knn: the listed rows are the matrix
+// itself (Q == nullptr) and a row is not its own neighbour. scema_query_knn: Q holds `rows` query rows of a second set,
+// and every one of the n rows is a candidate.
 struct Knn {
     scema_ctx *c;           // the caller's context: its stream, its rows, its scratch buffers
-    uint64_t n;
+    uint64_t n;             // rows of the caller's matrix: the candidate partners
+    uint64_t rows;          // rows whose neighbours are listed (n for scema_knn)
+    const double *Q = nullptr;
     uint32_t K, k;
     uint64_t open_n;        // rows still open
     std::vector<uint32_t> subset;
-    uint64_t stats[8] = {};
+    uint64_t stats[11] = {};
     double radii[8] = {};
 
     template <class T> T *buf(int b) { return c->knn_buf[b].as<T>(); }
@@ -278,18 +371,33 @@ struct Knn {
         SCEMA_CUDA(c, cudaStreamSynchronize(c->stream));
         return SCEMA_OK;
     }
+    uint64_t partners() const { return Q ? n : n - 1; }
+
+    // buffers, IDs of the candidate rows, every listed row open
+    int begin()
+    {
+        int rc;
+        if ((rc = reserve(B_IDS, n * sizeof(uint32_t))) || (rc = reserve(B_OPEN, rows)) || (rc = reserve(B_PERM, rows * sizeof(uint32_t))) ||
+            (rc = reserve(B_OUT_IX, rows * k * sizeof(uint32_t))) || (rc = reserve(B_OUT_D, rows * k * sizeof(double))) ||
+            (rc = reserve(B_MISC, 8 * sizeof(uint64_t))))
+            return rc;
+        SCEMA_CUDA(c, cudaMemcpyAsync(buf<void>(B_IDS), ids_of(c).data(), n * sizeof(uint32_t), cudaMemcpyHostToDevice, c->stream));
+        SCEMA_CUDA(c, cudaMemsetAsync(buf<void>(B_OPEN), 1, rows, c->stream));
+        open_n = rows;
+        return SCEMA_OK;
+    }
 
     // open rows first in B_PERM; returns their number in open_n
     int partition()
     {
         size_t tmp = 0;
         cub::CountingInputIterator<uint32_t> iota(0);
-        SCEMA_CUDA(c, cub::DevicePartition::Flagged(nullptr, tmp, iota, buf<uint8_t>(B_OPEN), buf<uint32_t>(B_PERM), misc() + 1, (int64_t)n,
+        SCEMA_CUDA(c, cub::DevicePartition::Flagged(nullptr, tmp, iota, buf<uint8_t>(B_OPEN), buf<uint32_t>(B_PERM), misc() + 1, (int64_t)rows,
                                                     c->stream));
         int rc = reserve(B_TMP, tmp);
         if (rc) return rc;
         SCEMA_CUDA(c, cub::DevicePartition::Flagged(buf<void>(B_TMP), tmp, iota, buf<uint8_t>(B_OPEN), buf<uint32_t>(B_PERM), misc() + 1,
-                                                    (int64_t)n, c->stream));
+                                                    (int64_t)rows, c->stream));
         c->launches += 2;
         uint64_t m[2];
         rc = read_misc(m, 2);
@@ -298,9 +406,9 @@ struct Knn {
         return SCEMA_OK;
     }
 
-    // Radius from a distance sample: A rows against the subset (round 1: the subset's own pairs). tau = the smallest
-    // value with at least max(C * k / (n - 1) * count, KNN_QUANTILE_MIN) sampled distances strictly below it; *frac_below =
-    // the sampled fraction below max(tau, floor). +inf (or 0 sampled distances) when no such value exists.
+    // Radius from a distance sample: A rows against the subset (round 1 of scema_knn: the subset's own pairs). tau = the
+    // smallest value with at least max(C * k / partners * count, KNN_QUANTILE_MIN) sampled distances strictly below it;
+    // *frac_below = the sampled fraction below max(tau, floor). +inf (or 0 sampled distances) when no such value exists.
     int radius(const uint32_t *rows_a, uint32_t na, uint64_t a_span, bool tri, double floor_tau, double *tau, double *frac_below)
     {
         const uint32_t nb = (uint32_t)subset.size();
@@ -309,8 +417,8 @@ struct Knn {
         if (rc) return rc;
         unsigned long long *s0 = buf<unsigned long long>(B_SAMPLE), *s1 = s0 + total;
         SCEMA_CUDA(c, cudaMemsetAsync(misc(), 0, 4 * sizeof(uint64_t), c->stream));
-        k_knn_sample<<<(unsigned)((total + 255) / 256), 256, 0, c->stream>>>(c->d_spline, K, rows_a, na, a_span, buf<uint32_t>(B_SUBSET), nb,
-                                                                           tri ? 1 : 0, s0, misc());
+        k_knn_sample<<<(unsigned)((total + 255) / 256), 256, 0, c->stream>>>(c->d_spline, Q ? Q : c->d_spline, Q ? 1 : 0, K, rows_a, na,
+                                                                           a_span, buf<uint32_t>(B_SUBSET), nb, tri ? 1 : 0, s0, misc());
         c->launches++;
         SCEMA_CUDA(c, cudaGetLastError());
         uint64_t count = 0;
@@ -326,7 +434,7 @@ struct Knn {
         if (rc) return rc;
         SCEMA_CUDA(c, cub::DeviceRadixSort::SortKeys(buf<void>(B_TMP), tmp, db, (int64_t)count, 0, 64, c->stream));
         c->launches += 17;
-        const double want = std::ceil(KNN_QUANTILE_C * k / (double)(n - 1) * (double)count);
+        const double want = std::ceil(KNN_QUANTILE_C * k / (double)partners() * (double)count);
         const uint64_t m = std::max<uint64_t>(KNN_QUANTILE_MIN, (uint64_t)std::min<double>(want, 1e18));
         if (m > count) return SCEMA_OK;
         double v = 0.0;
@@ -348,34 +456,35 @@ struct Knn {
     }
 
     // Close every open row that has at least k entries among the edges the child context holds (its matrix is the
-    // caller's rows in the order perm, nullptr = identity). Returns the rows closed.
-    int select(scema_ctx *child, const uint32_t *perm, uint64_t *closed)
+    // caller's rows in the order perm, nullptr = identity; with cross > 0 the first `cross` rows are the open queries in
+    // the order perm, then the caller's rows). Returns the rows closed.
+    int select(scema_ctx *child, const uint32_t *perm, uint64_t cross, uint64_t *closed)
     {
         const uint64_t m = child->n_edges;
         *closed = 0;
         if (m == 0) return SCEMA_OK;
         const uint64_t *keys = child->d_edge_key[child->edge_cur].as<uint64_t>();
         const double *vals = child->d_edge_val[child->edge_cur].as<double>();
-        int rc = reserve(B_CNT, 2 * (n + 1) * sizeof(unsigned long long));
+        int rc = reserve(B_CNT, 2 * (rows + 1) * sizeof(unsigned long long));
         if (!rc) rc = reserve(B_EB, 2 * m * sizeof(unsigned long long));
         if (!rc) rc = reserve(B_EIX, 2 * m * sizeof(uint32_t));
         if (rc) return rc;
-        unsigned long long *cnt = buf<unsigned long long>(B_CNT), *offs = cnt + (n + 1);
-        SCEMA_CUDA(c, cudaMemsetAsync(cnt, 0, (n + 1) * sizeof(unsigned long long), c->stream));
+        unsigned long long *cnt = buf<unsigned long long>(B_CNT), *offs = cnt + (rows + 1);
+        SCEMA_CUDA(c, cudaMemsetAsync(cnt, 0, (rows + 1) * sizeof(unsigned long long), c->stream));
         const unsigned g = (unsigned)((m + 255) / 256);
-        k_knn_expand<0><<<g, 256, 0, c->stream>>>(keys, vals, m, child->key_shift, perm, buf<uint8_t>(B_OPEN), cnt, nullptr, nullptr);
+        k_knn_expand<0><<<g, 256, 0, c->stream>>>(keys, vals, m, child->key_shift, perm, cross, buf<uint8_t>(B_OPEN), cnt, nullptr, nullptr);
         size_t tmp = 0;
-        SCEMA_CUDA(c, cub::DeviceScan::ExclusiveSum(nullptr, tmp, cnt, offs, (int64_t)(n + 1), c->stream));
+        SCEMA_CUDA(c, cub::DeviceScan::ExclusiveSum(nullptr, tmp, cnt, offs, (int64_t)(rows + 1), c->stream));
         rc = reserve(B_TMP, tmp);
         if (rc) return rc;
-        SCEMA_CUDA(c, cub::DeviceScan::ExclusiveSum(buf<void>(B_TMP), tmp, cnt, offs, (int64_t)(n + 1), c->stream));
-        SCEMA_CUDA(c, cudaMemcpyAsync(cnt, offs, (n + 1) * sizeof(unsigned long long), cudaMemcpyDeviceToDevice, c->stream));
-        k_knn_expand<1><<<g, 256, 0, c->stream>>>(keys, vals, m, child->key_shift, perm, buf<uint8_t>(B_OPEN), cnt,
+        SCEMA_CUDA(c, cub::DeviceScan::ExclusiveSum(buf<void>(B_TMP), tmp, cnt, offs, (int64_t)(rows + 1), c->stream));
+        SCEMA_CUDA(c, cudaMemcpyAsync(cnt, offs, (rows + 1) * sizeof(unsigned long long), cudaMemcpyDeviceToDevice, c->stream));
+        k_knn_expand<1><<<g, 256, 0, c->stream>>>(keys, vals, m, child->key_shift, perm, cross, buf<uint8_t>(B_OPEN), cnt,
                                                  buf<unsigned long long>(B_EB), buf<uint32_t>(B_EIX));
         SCEMA_CUDA(c, cudaMemsetAsync(misc() + 3, 0, sizeof(uint64_t), c->stream));
-        k_knn_topk<<<(unsigned)((n + 7) / 8), 256, 0, c->stream>>>(buf<unsigned long long>(B_EB), buf<uint32_t>(B_EIX), buf<uint32_t>(B_IDS),
-                                                                   nullptr, n, offs, 0, k, buf<uint8_t>(B_OPEN), misc() + 3,
-                                                                   buf<uint32_t>(B_OUT_IX), buf<double>(B_OUT_D));
+        k_knn_topk<<<(unsigned)((rows + 7) / 8), 256, 0, c->stream>>>(buf<unsigned long long>(B_EB), buf<uint32_t>(B_EIX), buf<uint32_t>(B_IDS),
+                                                                      nullptr, rows, offs, 0, k, buf<uint8_t>(B_OPEN), misc() + 3,
+                                                                      buf<uint32_t>(B_OUT_IX), buf<double>(B_OUT_D));
         c->launches += 5;
         SCEMA_CUDA(c, cudaGetLastError());
         uint64_t got[4];
@@ -399,33 +508,151 @@ struct Knn {
         int rc = reserve(B_PART_B, nq * nseg * k * sizeof(unsigned long long));
         if (!rc) rc = reserve(B_PART_IX, nq * nseg * k * sizeof(uint32_t));
         if (rc) return rc;
-        k_knn_exact<<<dim3((unsigned)qblocks, (unsigned)nseg), 256, 0, c->stream>>>(c->d_spline, n, K, buf<uint32_t>(B_IDS), buf<uint32_t>(B_PERM),
-                                                                                    (uint32_t)nq, seg_len, k, buf<unsigned long long>(B_PART_B),
-                                                                                    buf<uint32_t>(B_PART_IX));
+        k_knn_exact<<<dim3((unsigned)qblocks, (unsigned)nseg), 256, 0, c->stream>>>(c->d_spline, n, K, buf<uint32_t>(B_IDS), Q ? Q : c->d_spline,
+                                                                                    buf<uint32_t>(B_PERM), (uint32_t)nq, Q ? 0 : 1, seg_len, k,
+                                                                                    buf<unsigned long long>(B_PART_B), buf<uint32_t>(B_PART_IX));
         k_knn_topk<<<(unsigned)((nq + 7) / 8), 256, 0, c->stream>>>(buf<unsigned long long>(B_PART_B), buf<uint32_t>(B_PART_IX),
                                                                     buf<uint32_t>(B_IDS), buf<uint32_t>(B_PERM), nq, nullptr, nseg * k, k,
                                                                     nullptr, nullptr, buf<uint32_t>(B_OUT_IX), buf<double>(B_OUT_D));
         c->launches += 2;
         SCEMA_CUDA(c, cudaGetLastError());
         stats[3] += nq;
-        stats[4] += nq * (n - 1);
+        stats[4] += nq * partners();
+        return SCEMA_OK;
+    }
+
+    // Filter rounds on the private context `child`. Round 1 of scema_knn compares all rows at a radius from the subset's
+    // own pairs. Every other round (all rounds of scema_query_knn) samples the open rows against the subset, gathers them
+    // to the front of a scratch matrix — [open rows; the others] or [open queries; the caller's rows] — and compares the
+    // prefix panels that hold every pair involving them.
+    int rounds(scema_ctx *child, int variant)
+    {
+        make_subset(n, subset);
+        int rc = reserve(B_SUBSET, subset.size() * sizeof(uint32_t));
+        if (rc) return rc;
+        SCEMA_CUDA(c, cudaMemcpyAsync(buf<void>(B_SUBSET), subset.data(), subset.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, c->stream));
+        if (Q && (rc = partition())) return rc;  // B_PERM = the queries in order
+        const double budget = KNN_EDGE_BUDGET * (double)rows * k + 1048576.0;
+        double tau_prev = 0.0;
+        for (int round = 1; round <= KNN_MAX_ROUNDS && open_n > 0; round++) {
+            if (Q ? (double)open_n * (double)n <= KNN_QUERY_EXACT_PAIRS : (round > 1 && (double)open_n * (double)n <= KNN_EXACT_PAIRS)) break;
+            double tau = 0.0, frac = 1.0, pairs = 0.0;
+            uint32_t p1 = 0;
+            if (round == 1 && !Q) {
+                rc = radius(buf<uint32_t>(B_SUBSET), (uint32_t)subset.size(), subset.size(), true, 0.0, &tau, &frac);
+                pairs = 0.5 * (double)n * (double)(n - 1);
+            } else {
+                const uint32_t na = (uint32_t)std::min<uint64_t>(open_n, KNN_SAMPLE_OPEN);
+                rc = radius(buf<uint32_t>(B_PERM), na, open_n, false, 2.0 * tau_prev, &tau, &frac);
+                const uint32_t panel_rows = PANEL_ROWBLOCKS * TILE;
+                p1 = (uint32_t)((open_n + panel_rows - 1) / panel_rows);
+                const double N = Q ? (double)(open_n + n) : (double)n;
+                const double r1 = std::min<double>(N, (double)p1 * panel_rows);
+                pairs = r1 * N - 0.5 * r1 * (r1 + 1.0);
+            }
+            if (rc) return rc;
+            if (!(tau < INFINITY) || pairs * frac > budget) break;  // too dense for an O(rows k) edge list: the exact kernel takes over
+            const uint32_t *perm = nullptr;
+            const uint64_t cross = Q ? open_n : 0;
+            if (round == 1 && !Q) {
+                rc = scema_set_spline(child, c->d_spline, 1, n, K, nullptr);
+            } else {
+                QTimer t(c, QT_COPY, Q != nullptr);
+                const uint64_t lead = Q ? open_n : n;  // rows gathered through perm
+                if ((rc = reserve(B_ROWS, (cross + n) * K * sizeof(double)))) return rc;
+                k_knn_gather<<<(unsigned)((lead * K + 255) / 256), 256, 0, c->stream>>>(Q ? Q : c->d_spline, lead, K, buf<uint32_t>(B_PERM),
+                                                                                      buf<double>(B_ROWS));
+                c->launches++;
+                SCEMA_CUDA(c, cudaGetLastError());
+                if (Q)
+                    SCEMA_CUDA(c, cudaMemcpyAsync(buf<double>(B_ROWS) + cross * K, c->d_spline, n * K * sizeof(double), cudaMemcpyDeviceToDevice,
+                                                  c->stream));
+                t.stop();
+                rc = scema_set_spline(child, buf<double>(B_ROWS), 1, cross + n, K, nullptr);
+                perm = buf<uint32_t>(B_PERM);
+            }
+            if (rc) return fail(c, rc, std::string(Q ? "query_knn: " : "knn: ") + scema_last_error(child));
+            int v = variant;
+            rc = compare_prefix_run(child, tau, &v, p1, Q != nullptr);
+            if (rc) return fail(c, rc, std::string(Q ? "query_knn: " : "knn: ") + scema_last_error(child));
+            stats[0]++;
+            stats[5] += child->counters[1];
+            stats[6] += child->n_edges;
+            stats[7] = (uint64_t)v;
+            stats[8] += child->counters[0];
+            stats[10] += child->counters[3];
+            radii[round - 1] = tau;
+            tau_prev = tau;
+            if (Q) child_timings(child);
+            uint64_t closed = 0;
+            {
+                QTimer t(c, QT_SELECT, Q != nullptr);
+                rc = select(child, perm, cross, &closed);
+                if (rc) return rc;
+                stats[round == 1 ? 1 : 2] += closed;
+                rc = partition();  // the open rows to the front: sampled, gathered and queried by what follows
+                if (rc) return rc;
+                t.stop();
+            }
+        }
+        return SCEMA_OK;
+    }
+
+    // the child's phase timings of its last compare, added to the query's
+    void child_timings(scema_ctx *child)
+    {
+        float ms[SCEMA_T_COUNT];
+        if (scema_last_timings(child, ms) == SCEMA_OK)
+            for (int w = SCEMA_T_PREP; w <= SCEMA_T_SORT; w++) c->query_ms[QT_PREP + (w - SCEMA_T_PREP)] += ms[w];
+    }
+
+    // the open rows to the exact kernel, results to the host
+    int finish(uint32_t *index_host, double *diff_host)
+    {
+        int rc = partition();
+        if (rc) return rc;
+        {
+            QTimer t(c, QT_TOPK, Q != nullptr);
+            rc = exact();
+            if (rc) return rc;
+            t.stop();
+        }
+        if (index_host)
+            SCEMA_CUDA(c, cudaMemcpyAsync(index_host, buf<void>(B_OUT_IX), rows * k * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+        if (diff_host)
+            SCEMA_CUDA(c, cudaMemcpyAsync(diff_host, buf<void>(B_OUT_D), rows * k * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+        SCEMA_CUDA(c, cudaStreamSynchronize(c->stream));
         return SCEMA_OK;
     }
 };
 
-// Seeded stratified subset: one row from each of S equal slices of [0, n).
-void make_subset(uint64_t n, std::vector<uint32_t> &out)
+// private context (same device and stream) for the compares of a query call
+int child_of(scema_ctx *ctx, scema_ctx **slot, const char *what)
 {
-    const uint64_t s = std::min<uint64_t>(n, KNN_SAMPLE_ROWS);
-    out.resize(s);
-    for (uint64_t i = 0; i < s; i++) {
-        uint64_t z = KNN_SEED + 0x9e3779b97f4a7c15ull * (i + 1);
-        z = (z ^ (z >> 30)) * 0xbf58476d1ce4e5b9ull;
-        z = (z ^ (z >> 27)) * 0x94d049bb133111ebull;
-        z ^= z >> 31;
-        const uint64_t lo = i * n / s, hi = (i + 1) * n / s;
-        out[i] = (uint32_t)(lo + z % (hi - lo));
+    if (!*slot) {
+        scema_ctx *child = nullptr;
+        const int rc = scema_create(&child, ctx->device, (void *)ctx->stream);
+        if (rc) return fail(ctx, rc, std::string(what) + ": could not create the context of the filter rounds");
+        *slot = child;
     }
+    return SCEMA_OK;
+}
+
+// checks shared by scema_query_compare and scema_query_knn; resets the stats of the last query
+int query_check(scema_ctx *ctx, const double *rows, uint64_t m, uint32_t k_cols, int variant, const char *what)
+{
+    for (int i = 0; i < 11; i++) ctx->query_counts[i] = 0;
+    for (int i = 0; i < 8; i++) { ctx->query_radii[i] = 0.0; ctx->query_ms[i] = 0.f; }
+    ctx->query_counts[7] = SCEMA_PAIRS_EXACT;
+    if (!ctx->have_spline) return fail(ctx, SCEMA_ERR_STATE, "Spline is not up to date.");
+    if (k_cols != ctx->K) return fail(ctx, SCEMA_ERR_INVALID, std::string(what) + ": query rows must have as many columns as the spline matrix");
+    if (variant < 0 || variant > 3) return fail(ctx, SCEMA_ERR_INVALID, std::string(what) + ": bad variant");
+    if (m > 0 && !rows) return fail(ctx, SCEMA_ERR_INVALID, std::string(what) + ": null pointer");
+    if (m >= (1ull << 32) || ctx->n + m >= (1ull << 32)) return fail(ctx, SCEMA_ERR_INVALID, std::string(what) + ": n + m must stay below 2^32");
+    if (!ctx->query_ev[0]) {
+        for (int e = 0; e < 2; e++) SCEMA_CUDA(ctx, cudaEventCreate(&ctx->query_ev[e]));
+    }
+    return SCEMA_OK;
 }
 
 }  // namespace
@@ -439,7 +666,7 @@ int knn_run(scema_ctx *ctx, uint32_t k, int variant, uint32_t *index_host, doubl
     if (ctx->n >= (1ull << 32)) return fail(ctx, SCEMA_ERR_INVALID, "knn: more than 2^32-1 histories");
     const uint64_t n = ctx->n;
     Knn q;
-    q.c = ctx; q.n = n; q.K = ctx->K; q.k = k;
+    q.c = ctx; q.n = n; q.rows = n; q.K = ctx->K; q.k = k;
     q.stats[7] = SCEMA_PAIRS_EXACT;
     if (n <= 1) {
         if (index_host) std::fill(index_host, index_host + n * k, 0xffffffffu);
@@ -449,85 +676,124 @@ int knn_run(scema_ctx *ctx, uint32_t k, int variant, uint32_t *index_host, doubl
         return SCEMA_OK;
     }
     int rc = wait_rows(ctx);
+    if (!rc) rc = q.begin();
     if (rc) return rc;
-    if ((rc = q.reserve(B_IDS, n * sizeof(uint32_t))) || (rc = q.reserve(B_OPEN, n)) || (rc = q.reserve(B_PERM, n * sizeof(uint32_t))) ||
-        (rc = q.reserve(B_OUT_IX, n * k * sizeof(uint32_t))) || (rc = q.reserve(B_OUT_D, n * k * sizeof(double))) ||
-        (rc = q.reserve(B_MISC, 8 * sizeof(uint64_t))))
-        return rc;
-    SCEMA_CUDA(ctx, cudaMemcpyAsync(q.buf<void>(B_IDS), ids_of(ctx).data(), n * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
-    SCEMA_CUDA(ctx, cudaMemsetAsync(q.buf<void>(B_OPEN), 1, n, ctx->stream));
-    q.open_n = n;
-
     if (variant != SCEMA_PAIRS_EXACT && n >= KNN_MIN_N) {
-        if (!ctx->knn_child) {
-            scema_ctx *child = nullptr;
-            rc = scema_create(&child, ctx->device, (void *)ctx->stream);
-            if (rc) return fail(ctx, rc, "knn: could not create the context of the filter rounds");
-            ctx->knn_child = child;
-        }
-        scema_ctx *child = ctx->knn_child;
-        make_subset(n, q.subset);
-        if ((rc = q.reserve(B_SUBSET, q.subset.size() * sizeof(uint32_t)))) return rc;
-        SCEMA_CUDA(ctx, cudaMemcpyAsync(q.buf<void>(B_SUBSET), q.subset.data(), q.subset.size() * sizeof(uint32_t), cudaMemcpyHostToDevice,
-                                        ctx->stream));
-        const double budget = KNN_EDGE_BUDGET * (double)n * k + 1048576.0;
-        double tau_prev = 0.0;
-        for (int round = 1; round <= KNN_MAX_ROUNDS && q.open_n > 0; round++) {
-            if (round > 1 && (double)q.open_n * (double)n <= KNN_EXACT_PAIRS) break;
-            double tau = 0.0, frac = 1.0, pairs = 0.0;
-            uint32_t p1 = 0;
-            if (round == 1) {
-                rc = q.radius(q.buf<uint32_t>(B_SUBSET), (uint32_t)q.subset.size(), q.subset.size(), true, 0.0, &tau, &frac);
-                pairs = 0.5 * (double)n * (double)(n - 1);
-            } else {
-                const uint32_t na = (uint32_t)std::min<uint64_t>(q.open_n, KNN_SAMPLE_OPEN);
-                rc = q.radius(q.buf<uint32_t>(B_PERM), na, q.open_n, false, 2.0 * tau_prev, &tau, &frac);
-                const uint32_t panel_rows = PANEL_ROWBLOCKS * TILE;
-                p1 = (uint32_t)((q.open_n + panel_rows - 1) / panel_rows);
-                const double r1 = std::min<double>((double)n, (double)p1 * panel_rows);
-                pairs = r1 * (double)n - 0.5 * r1 * (r1 + 1.0);
-            }
-            if (rc) return rc;
-            if (!(tau < INFINITY) || pairs * frac > budget) break;  // too dense for an O(n k) edge list: the exact kernel takes over
-            const uint32_t *perm = nullptr;
-            if (round == 1) {
-                rc = scema_set_spline(child, ctx->d_spline, 1, n, q.K, nullptr);
-            } else {
-                if ((rc = q.reserve(B_ROWS, n * q.K * sizeof(double)))) return rc;
-                k_knn_gather<<<(unsigned)((n * q.K + 255) / 256), 256, 0, ctx->stream>>>(ctx->d_spline, n, q.K, q.buf<uint32_t>(B_PERM),
-                                                                                        q.buf<double>(B_ROWS));
-                ctx->launches++;
-                SCEMA_CUDA(ctx, cudaGetLastError());
-                rc = scema_set_spline(child, q.buf<double>(B_ROWS), 1, n, q.K, nullptr);
-                perm = q.buf<uint32_t>(B_PERM);
-            }
-            if (rc) return fail(ctx, rc, std::string("knn: ") + scema_last_error(child));
-            int v = variant;
-            rc = compare_prefix_run(child, tau, &v, p1);
-            if (rc) return fail(ctx, rc, std::string("knn: ") + scema_last_error(child));
-            q.stats[0]++;
-            q.stats[5] += child->counters[1];
-            q.stats[6] += child->n_edges;
-            q.stats[7] = (uint64_t)v;
-            q.radii[round - 1] = tau;
-            tau_prev = tau;
-            uint64_t closed = 0;
-            rc = q.select(child, perm, &closed);
-            if (rc) return rc;
-            q.stats[round == 1 ? 1 : 2] += closed;
-            rc = q.partition();  // the open rows to the front: sampled, gathered and queried by what follows
-            if (rc) return rc;
-        }
+        if ((rc = child_of(ctx, &ctx->knn_child, "knn")) || (rc = q.rounds(ctx->knn_child, variant))) return rc;
     }
-    rc = q.partition();
-    if (!rc) rc = q.exact();
-    if (rc) return rc;
-    if (index_host)
-        SCEMA_CUDA(ctx, cudaMemcpyAsync(index_host, q.buf<void>(B_OUT_IX), n * k * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
-    if (diff_host)
-        SCEMA_CUDA(ctx, cudaMemcpyAsync(diff_host, q.buf<void>(B_OUT_D), n * k * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-    SCEMA_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    if ((rc = q.finish(index_host, diff_host))) return rc;
     for (int i = 0; i < 8; i++) { ctx->knn_counts[i] = q.stats[i]; ctx->knn_radii[i] = q.radii[i]; }
+    return SCEMA_OK;
+}
+
+int query_knn_run(scema_ctx *ctx, const double *rows, int rows_on_device, uint64_t m, uint32_t k_cols, uint32_t k, int variant,
+                  uint32_t *index_host, double *diff_host)
+{
+    int rc = query_check(ctx, rows, m, k_cols, variant, "query_knn");
+    if (rc) return rc;
+    if (k < 1 || k > 32) return fail(ctx, SCEMA_ERR_INVALID, "query_knn: k must be in [1, 32]");
+    const uint64_t n = ctx->n;
+    if (m == 0) return SCEMA_OK;
+    if (n == 0) {
+        if (index_host) std::fill(index_host, index_host + m * k, 0xffffffffu);
+        if (diff_host) std::fill(diff_host, diff_host + m * k, INFINITY);
+        ctx->query_counts[3] = m;
+        return SCEMA_OK;
+    }
+    Knn q;
+    q.c = ctx; q.n = n; q.rows = m; q.K = ctx->K; q.k = k;
+    q.stats[7] = SCEMA_PAIRS_EXACT;
+    if ((rc = wait_rows(ctx))) return rc;
+    q.Q = rows;
+    if (!rows_on_device) {
+        QTimer t(ctx, QT_COPY, true);  // the upload of host queries counts as scratch copy, as in scema_query_compare
+        if ((rc = q.reserve(B_Q, m * q.K * sizeof(double)))) return rc;
+        SCEMA_CUDA(ctx, cudaMemcpyAsync(q.buf<void>(B_Q), rows, m * q.K * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+        t.stop();
+        q.Q = q.buf<double>(B_Q);
+    }
+    if ((rc = q.begin())) return rc;
+    if (variant != SCEMA_PAIRS_EXACT) {
+        if ((rc = child_of(ctx, &ctx->query_child, "query_knn")) || (rc = q.rounds(ctx->query_child, variant))) return rc;
+    }
+    if ((rc = q.finish(index_host, diff_host))) return rc;
+    for (int i = 0; i < 11; i++) ctx->query_counts[i] = q.stats[i];
+    for (int i = 0; i < 8; i++) ctx->query_radii[i] = q.radii[i];
+    return SCEMA_OK;
+}
+
+// scema_query_compare: [Q; R] on the private context, the prefix panels [0, ceil(m / 2048)) compared (they hold every
+// query x retained pair), the cross edges compacted into the context's query buffers.
+int query_compare_run(scema_ctx *ctx, const double *rows, int rows_on_device, uint64_t m, uint32_t k_cols, double thr, int variant,
+                      uint64_t *n_edges)
+{
+    ctx->have_query = false;
+    ctx->query_n = 0;
+    if (n_edges) *n_edges = 0;
+    int rc = query_check(ctx, rows, m, k_cols, variant, "query_compare");
+    if (rc) return rc;
+    ctx->query_radii[0] = thr;
+    const uint64_t n = ctx->n, K = ctx->K, N = m + n;
+    if (m == 0 || n == 0 || !(thr > 0.0)) {  // diff >= 0 or NaN: nothing passes a non-positive or NaN threshold
+        ctx->have_query = true;
+        return SCEMA_OK;
+    }
+    if ((rc = wait_rows(ctx)) || (rc = child_of(ctx, &ctx->query_child, "query_compare"))) return rc;
+    scema_ctx *child = ctx->query_child;
+    DevBuf &stack = ctx->knn_buf[B_ROWS];
+    {
+        QTimer t(ctx, QT_COPY, true);
+        SCEMA_CUDA(ctx, stack.reserve(N * K * sizeof(double)));
+        SCEMA_CUDA(ctx, cudaMemcpyAsync(stack.p, rows, m * K * sizeof(double), rows_on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice,
+                                        ctx->stream));
+        SCEMA_CUDA(ctx, cudaMemcpyAsync(stack.as<double>() + m * K, ctx->d_spline, n * K * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
+        t.stop();
+    }
+    rc = scema_set_spline(child, stack.as<double>(), 1, N, (uint32_t)K, nullptr);
+    if (rc) return fail(ctx, rc, std::string("query_compare: ") + scema_last_error(child));
+    const uint32_t panel_rows = PANEL_ROWBLOCKS * TILE;
+    int v = variant;
+    rc = compare_prefix_run(child, thr, &v, (uint32_t)((m + panel_rows - 1) / panel_rows), true);
+    if (rc) return fail(ctx, rc, std::string("query_compare: ") + scema_last_error(child));
+    Knn q;  // scratch buffers only
+    q.c = ctx;
+    const uint64_t ne = child->n_edges;
+    uint64_t kept = 0;
+    if (ne) {
+        QTimer t(ctx, QT_SELECT, true);
+        const uint64_t *keys = child->d_edge_key[child->edge_cur].as<uint64_t>();
+        const double *vals = child->d_edge_val[child->edge_cur].as<double>();
+        if ((rc = q.reserve(B_CNT, 2 * (ne + 1) * sizeof(unsigned long long)))) return rc;
+        unsigned long long *flag = q.buf<unsigned long long>(B_CNT), *pos = flag + (ne + 1);
+        k_query_flag<<<(unsigned)((ne + 1 + 255) / 256), 256, 0, ctx->stream>>>(keys, ne, child->key_shift, m, flag);
+        size_t tmp = 0;
+        SCEMA_CUDA(ctx, cub::DeviceScan::ExclusiveSum(nullptr, tmp, flag, pos, (int64_t)(ne + 1), ctx->stream));
+        if ((rc = q.reserve(B_TMP, tmp))) return rc;
+        SCEMA_CUDA(ctx, cub::DeviceScan::ExclusiveSum(q.buf<void>(B_TMP), tmp, flag, pos, (int64_t)(ne + 1), ctx->stream));
+        SCEMA_CUDA(ctx, cudaMemcpyAsync(&kept, pos + ne, sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
+        SCEMA_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        SCEMA_CUDA(ctx, ctx->query_j.reserve(std::max<uint64_t>(kept, 1) * sizeof(uint32_t)));
+        SCEMA_CUDA(ctx, ctx->query_i.reserve(std::max<uint64_t>(kept, 1) * sizeof(uint32_t)));
+        SCEMA_CUDA(ctx, ctx->query_d.reserve(std::max<uint64_t>(kept, 1) * sizeof(double)));
+        k_query_scatter<<<(unsigned)((ne + 255) / 256), 256, 0, ctx->stream>>>(keys, vals, ne, child->key_shift, m, flag, pos,
+                                                                               ctx->query_j.as<uint32_t>(), ctx->query_i.as<uint32_t>(),
+                                                                               ctx->query_d.as<double>());
+        ctx->launches += 4;
+        SCEMA_CUDA(ctx, cudaGetLastError());
+        t.stop();
+    }
+    q.child_timings(child);
+    uint64_t *st = ctx->query_counts;
+    st[0] = 1;
+    st[5] = child->counters[1];
+    st[6] = ne;
+    st[7] = (uint64_t)v;
+    st[8] = child->counters[0];
+    st[9] = kept;
+    st[10] = child->counters[3];
+    ctx->query_n = kept;
+    ctx->have_query = true;
+    if (n_edges) *n_edges = kept;
     return SCEMA_OK;
 }
 

@@ -1216,8 +1216,9 @@ int edges_adopt(scema_ctx *ctx, const uint64_t *d_keys, const double *d_vals, ui
 }
 
 // Common front end: argument checks, buffers, filter copy and schedule. Returns 1 when there is
-// nothing to compare (result: no edges).
-static int compare_begin(scema_ctx *ctx, double thr, int &variant, uint32_t shard, uint32_t n_shards, Schedule &sc)
+// nothing to compare (result: no edges). plan_pairs: the pairs the filter choice is made for (0: this shard's share of
+// the whole triangle).
+static int compare_begin(scema_ctx *ctx, double thr, int &variant, uint32_t shard, uint32_t n_shards, Schedule &sc, uint64_t plan_pairs = 0)
 {
     if (!ctx->have_spline) return fail(ctx, SCEMA_ERR_STATE, "Spline is not up to date.");
     if (n_shards == 0 || shard >= n_shards) return fail(ctx, SCEMA_ERR_INVALID, "compare: bad shard");
@@ -1259,7 +1260,7 @@ static int compare_begin(scema_ctx *ctx, double thr, int &variant, uint32_t shar
         const bool want_band = ctx->tc_band_allowed && band_env && atoi(band_env) == 1;
         int choice = 1;
         uint64_t est = 0;
-        rc = tc_prepare(ctx, thr, slices, want_band, n * (n - 1) / 2 / n_shards, &choice, &est);
+        rc = tc_prepare(ctx, thr, slices, want_band, plan_pairs ? plan_pairs : n * (n - 1) / 2 / n_shards, &choice, &est);
         if (rc) return rc;
         if (choice == 0) variant = SCEMA_PAIRS_DMMA;
         else if (choice < 0) variant = SCEMA_PAIRS_EXACT;
@@ -1278,16 +1279,28 @@ static int compare_begin(scema_ctx *ctx, double thr, int &variant, uint32_t shar
     return SCEMA_OK;
 }
 
-// The rounds of scema_knn (knn.cu): every pair (a, b), a < b, with a in the row panels [0, p1) (p1 = 0: all of them),
-// one GPU, no audit. The edges are left as after compare_run; *variant becomes the filter that ran.
-int compare_prefix_run(scema_ctx *ctx, double thr, int *variant, uint32_t p1)
+// pairs (a, b), a < b, with a in the row panels [0, p1) of n rows
+static uint64_t prefix_pairs(uint64_t n, uint32_t p1)
+{
+    const uint64_t r1 = std::min<uint64_t>(n, (uint64_t)p1 * PANEL_ROWBLOCKS * TILE);
+    return r1 * n - r1 * (r1 + 1) / 2;
+}
+
+// The rounds of scema_knn and the scema_query_* calls (knn.cu): every pair (a, b), a < b, with a in the row panels
+// [0, p1) (p1 = 0: all of them), one GPU, no audit. plan_prefix: the filter is chosen for the pairs of those panels (a
+// small query in front of a large matrix must not be planned as the whole triangle: that overestimates its survivors by
+// up to (n + m) / 2m); otherwise for the whole triangle, as scema_knn does. The edges are left as after compare_run,
+// counters[0] = the pairs of the panels; *variant becomes the filter that ran.
+int compare_prefix_run(scema_ctx *ctx, double thr, int *variant, uint32_t p1, bool plan_prefix)
 {
     Schedule sc;
-    int rc = compare_begin(ctx, thr, *variant, 0, 1, sc);
+    int rc = compare_begin(ctx, thr, *variant, 0, 1, sc, plan_prefix && p1 ? prefix_pairs(ctx->n, p1) : 0);
     if (rc < 0) return SCEMA_OK;
     if (rc) return rc;
-    rc = compare_panels(ctx, thr, variant, 0, 1, sc, 0, p1 ? std::min<uint32_t>(p1, sc.n_panels) : sc.n_panels);
+    const uint32_t p_end = p1 ? std::min<uint32_t>(p1, sc.n_panels) : sc.n_panels;
+    rc = compare_panels(ctx, thr, variant, 0, 1, sc, 0, p_end);
     if (rc) return rc;
+    ctx->counters[0] = prefix_pairs(ctx->n, p_end);
     ctx->counters[2] = ctx->n_edges;
     return SCEMA_OK;
 }
